@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the CISTA-Flow motion-compensation hot path (driver contract).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 Headline workload = BASELINE.json configs[4]: 64 independent 480x640 event sequences, cista-eiflow
 shape, STRONG-scaled over the N GPUs of one box (64/N streams per rank, no data-path collective).
@@ -25,6 +25,9 @@ cpu_baseline / --impl reference   the oracle port of the reference's own CPU pat
            CPU calls the reference makes) on a bounded sample of the same workload, all host threads.
 other_configs   (N=1 only) configs[0] B=1 latency, configs[1] (round 1's headline), configs[2] the
            260x346 voxel+warp microbench at x1/x64/x1024 windows, configs[3] 624x970 / 1 M events.
+--dump-outputs DIR   after the timed steps, what the last timed step returned (voxel grids, every lookup output, warped
+           frame and codes; rank 0) as DIR/<name>.npy, float32, a fixed sample of each output (see dump_outputs).  The
+           inputs are seeded, so two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -35,6 +38,9 @@ import statistics
 import subprocess
 import sys
 import time
+
+# the tree may be read-only: no __pycache__ next to the sources
+sys.dont_write_bytecode = True
 
 # torchrun exports OMP_NUM_THREADS=1 to every rank; the CPU reference arm (rank 0) must get all host cores
 if os.environ.get("OMP_NUM_THREADS") == "1" and os.environ.get("RANK", "0") == "0":
@@ -248,6 +254,7 @@ def cpu_step(cfg, host, ids):
 
 
 def time_cpu(cfg, host, sample, steps, warmup):
+    """(seconds per step, host threads, what the last step returned)"""
     try:
         os.sched_setaffinity(0, range(os.cpu_count() or 1))
     except OSError:
@@ -259,9 +266,28 @@ def time_cpu(cfg, host, sample, steps, warmup):
         cpu_step(cfg, host, ids)
     t0 = time.perf_counter()
     for _ in range(steps):
-        cpu_step(cfg, host, ids)
+        last = cpu_step(cfg, host, ids)
     dt = time.perf_counter() - t0
-    return dt / steps, torch.get_num_threads()
+    return dt / steps, torch.get_num_threads(), last
+
+
+DUMP_BYTES = 48 << 20   # all files --dump-outputs writes, together
+
+
+def dump_outputs(out_dir, grids, outs, wi, wz):
+    """One step's results (voxel grids, lookup outputs, warped frame, warped codes) as out_dir/<name>.npy, float32.
+    An output larger than its share of DUMP_BYTES is stored as its elements at a fixed sample of flat indices (sorted,
+    NumPy default_rng(0)): the same positions on every run of the same workload."""
+    arrays = {"voxel": torch.as_tensor(np.stack(grids)) if isinstance(grids, list) else grids,
+              **{f"lookup{k}": o for k, o in enumerate(outs)}, "warped_frame": wi, "warped_codes": wz}
+    cap = DUMP_BYTES // 4 // len(arrays)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        t = t.reshape(-1)
+        if t.numel() > cap:
+            idx = np.sort(np.random.default_rng(0).integers(0, t.numel(), cap))
+            t = t[torch.from_numpy(idx).to(t.device)]
+        np.save(os.path.join(out_dir, name + ".npy"), t.float().cpu().numpy())
 
 
 def run_reference(args, cfg):
@@ -271,7 +297,9 @@ def run_reference(args, cfg):
         return  # the CPU arm runs on rank 0 only
     sample = 4  # streams per step: a bounded sample of the 64-stream job (one 480x640 stream-frame is ~0.25 s on 8 cores)
     host = make_host_streams(cfg, 1234 + 1000 * 4, sample)
-    sec, cores = time_cpu(cfg, host, sample, args.steps, args.warmup)
+    sec, cores, last = time_cpu(cfg, host, sample, args.steps, args.warmup)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, *last)
     fps = sample / sec
     desc = (f"each step = the full hot path of {sample} of the 64 streams (480x640, 100000 events, 6 lookups) through "
             f"oracle/ref_port.py (the reference's own NumPy/torch CPU calls), {args.steps} steps after {args.warmup} "
@@ -605,6 +633,8 @@ def run_ours(args, cfg):
         sampler = ClockSampler(local_rank) if rank == 0 else None
         step_ms_local = time_graphs(graphs, stream, args.steps, args.warmup, barrier)
         other_form_ms_local = cal[not branched]
+        if args.dump_outputs and rank == 0:     # replay i used graphs[i % n]: keep[(steps - 1) % n] holds the last step
+            dump_outputs(args.dump_outputs, *keep[(args.steps - 1) % len(keep)])
 
         # -- e2e: pinned host buffers -> H2D -> public API (the captured graph) -> D2H, every step.  Three streams
         #    (upload / compute / read-back) over the two device buffer sets, so the PCIe transfers of neighbouring
@@ -650,7 +680,7 @@ def run_ours(args, cfg):
                     dst.copy_(src, non_blocking=True)
                 ev_d2h[k].record(s_d2h)
 
-        e2e_steps = max(4, min(args.steps, 20))
+        e2e_steps = args.steps
         for i in range(max(3, n_sets)):
             e2e_step(i)
         barrier()
@@ -726,11 +756,11 @@ def run_ours(args, cfg):
             other = {}
             with torch.cuda.stream(stream):
                 for name in ("configs[0]", "configs[1]", "configs[3]"):
-                    other[name] = other_config_line(name, dev, stream, hbm, tf32_peak, steps=20)
+                    other[name] = other_config_line(name, dev, stream, hbm, tf32_peak, steps=args.steps)
                 other["configs[2]"] = microbench_config2(dev, stream, hbm)
         sample = 4
         host = make_host_streams(cfg, 1234 + 1000 * 4, sample)
-        sec, cores = time_cpu(cfg, host, sample, steps=3, warmup=1)
+        sec, cores, _ = time_cpu(cfg, host, sample, steps=3, warmup=1)
         cpu = {"value": sample / sec, "unit": "frames/s", "cores": cores, "kind": "port", "ms_per_step": sec * 1e3,
                "sample": f"3 steps after 1 warm-up, each the full hot path of {sample} of the 64 streams (480x640, 100000 "
                          f"events, 6 lookups), oracle/ref_port.py (the reference's own NumPy/torch CPU calls), all host threads"}
@@ -801,7 +831,10 @@ def main():
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--impl", choices=["ours", "reference"], default="ours")
     ap.add_argument("--no-extra", action="store_true", help="skip the other BASELINE configs (N=1 extras)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step computed to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3)
     cfg = make_cfg("configs[4]")
     if args.impl == "reference":
@@ -815,6 +848,8 @@ def main():
                    "--gpus", str(args.gpus), "--steps", str(args.steps), "--warmup", str(args.warmup)]
             if args.no_extra:
                 cmd.append("--no-extra")
+            if args.dump_outputs:
+                cmd += ["--dump-outputs", args.dump_outputs]
             sys.exit(subprocess.call(cmd))
         run_ours(args, cfg)
 

@@ -15,6 +15,33 @@ def pytest_configure(config):
     config.addinivalue_line("markers", "gpu: needs a CUDA device (B200); run with `-m gpu` on the GPU box")
 
 
+class Fixture(dict):
+    """The arrays of one fixture.  An array stored as a fixed sample (KEY#values / KEY#mask / KEY#shape, see
+    tests/golden/make_golden.py) is expanded to a zero-filled array of its full shape; ``pick`` restricts a computed
+    output and the stored one to the sampled elements."""
+
+    def __init__(self, z):
+        super().__init__()
+        self.masks = {}
+        for k in z.files:
+            if k.endswith("#values"):
+                key = k[: -len("#values")]
+                shape = tuple(int(s) for s in z[key + "#shape"])
+                mask = np.unpackbits(z[key + "#mask"], count=int(np.prod(shape))).astype(bool).reshape(shape)
+                full = np.zeros(shape, z[k].dtype)
+                full[mask] = z[k]
+                self[key], self.masks[key] = full, mask
+            elif "#" not in k:
+                self[k] = z[k]
+
+    def pick(self, key, got):
+        """(got, stored) where the fixture stores ``key``."""
+        got, ref = np.asarray(got), self[key]
+        assert got.shape == ref.shape, (key, got.shape, ref.shape)
+        mask = self.masks.get(key)
+        return (got, ref) if mask is None else (got[mask], ref[mask])
+
+
 @pytest.fixture(scope="session")
 def golden():
     """Loader for the fixtures generated from the reference (tests/golden/make_golden.py)."""
@@ -23,7 +50,7 @@ def golden():
     def load(name):
         if name not in cache:
             with np.load(os.path.join(GOLDEN, name + ".npz")) as z:
-                cache[name] = {k: z[k] for k in z.files}
+                cache[name] = Fixture(z)
         return cache[name]
     return load
 

@@ -1,12 +1,11 @@
 #!/usr/bin/env python
 """Generate golden input/output fixtures from the REFERENCE ITSELF.
 
-Run in the build container only (``/root/reference`` does not exist on the GPU
-box and no test reads it at run time):
+Run with a checkout of the original project (no test reads it at run time):
 
-    PYTHONDONTWRITEBYTECODE=1 python tests/golden/make_golden.py
+    CISTA_REFERENCE=<checkout> PYTHONDONTWRITEBYTECODE=1 python tests/golden/make_golden.py
 
-The reference is imported read-only from ``/root/reference``; every array stored
+The reference is imported read-only from ``$CISTA_REFERENCE``; every array stored
 below is either a seeded synthetic input or the output of an unmodified
 reference function on that input.  The reference has no tests or golden vectors
 of its own (SURVEY.md F3), so these files are what pins the oracle.
@@ -36,7 +35,7 @@ import types
 import numpy as np
 import torch
 
-REF = os.environ.get("CISTA_REFERENCE", "/root/reference")
+REF = os.environ.get("CISTA_REFERENCE", "")
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(os.path.dirname(HERE))
 sys.dont_write_bytecode = True
@@ -66,8 +65,117 @@ def _stub_optional_imports():
 
 def save(name, **arrays):
     path = os.path.join(HERE, name)
+    arrays = compact(name, arrays)
     np.savez_compressed(path, **arrays)
     print(f"{name}: {os.path.getsize(path) / 1024:.0f} KiB, {len(arrays)} arrays")
+
+
+# ---------------------------------------------------------------- sampling ---
+# Every fixture stays below 1 MB.  The correlation, trace and multi-frame trace fixtures therefore keep a fixed sample
+# of their large arrays: KEY#values holds the elements at the set bits of KEY#mask (np.packbits of a boolean array of
+# shape KEY#shape); tests/conftest.py expands them to zero-filled arrays of the full shape, and the tests compare
+# outputs only where the fixture stores them.  A sample is chosen so that the stored outputs depend only on stored
+# inputs: a correlation row depends on its query's fmap1 column and all of fmap2, a lookup on its query's rows, a warped
+# pixel on the flow there and on the source within MARGIN pixels (|flow| < 10 px in these traces), a warped code channel
+# on that channel alone.  Event streams that synth.events() regenerates from a seed are stored as the seed.
+MARGIN = 12
+
+
+def _sparse(out, key, keep):
+    a = out.pop(key)
+    keep = np.broadcast_to(keep, a.shape)
+    out[key + "#shape"] = np.array(a.shape)
+    out[key + "#mask"] = np.packbits(keep.ravel())
+    out[key + "#values"] = a[keep]
+
+
+def _queries(rng, b, h, w, frac, extra=()):
+    """Sampled correlation queries, bool [b, h, w]."""
+    q = rng.random((b, h, w)) < frac
+    for idx in extra:
+        q[idx] = True
+    return q
+
+
+def _rows(q):
+    """Pyramid level [b*h*w, 1, hl, wl]: the rows of the sampled queries."""
+    return q.reshape(-1, 1, 1, 1)
+
+
+def _positions(q):
+    """[b, c, h, w] maps (fmap1, lookup outputs): every channel at the sampled queries."""
+    return q[:, None]
+
+
+def _box(shape, r0, r1, c0, c1, channels=None):
+    """[b, c, h, w]: rows r0:r1, columns c0:c1 (clipped to the map), channels :channels."""
+    keep = np.zeros(shape, bool)
+    keep[:, :channels, max(r0, 0):r1, max(c0, 0):c1] = True
+    return keep
+
+
+def _warp_boxes(out, h, w, frame_in, frame_out, flows, codes_in, codes_out, half_flow, channels):
+    """Frame warp: outputs in the central box (a third of each side), flow there (+4 px for the x0.5 down-sampling),
+    source within MARGIN.  Codes warp (half resolution): outputs in that box halved and shrunk by 2 px, the first
+    `channels` channels."""
+    r0, r1, c0, c1 = h // 3, 2 * h // 3, w // 3, 2 * w // 3
+    _sparse(out, frame_out, _box(out[frame_out].shape, r0, r1, c0, c1))
+    _sparse(out, frame_in, _box(out[frame_in].shape, r0 - MARGIN, r1 + MARGIN, c0 - MARGIN, c1 + MARGIN))
+    for key in flows:
+        _sparse(out, key, _box(out[key].shape, r0 - 4, r1 + 4, c0 - 4, c1 + 4))
+    s0, s1, t0, t1 = r0 // 2 + 2, r1 // 2 - 2, c0 // 2 + 2, c1 // 2 - 2
+    _sparse(out, codes_out, _box(out[codes_out].shape, s0, s1, t0, t1, channels))
+    _sparse(out, codes_in, _box(out[codes_in].shape, s0 - MARGIN, s1 + MARGIN, t0 - MARGIN, t1 + MARGIN, channels))
+    if half_flow:
+        _sparse(out, half_flow, _box(out[half_flow].shape, s0, s1, t0, t1))
+
+
+def compact(name, out):
+    out = dict(out)
+    rng = np.random.default_rng(0)
+    if name == "corr.npz":
+        q = _queries(rng, 1, 16, 24, 0.25, extra=[(0, 0, 0), (0, 1, 1)])   # the two hand-placed queries
+        for l in range(4):
+            _sparse(out, f"pyr{l}", _rows(q))
+        _sparse(out, "lookup", _positions(q))
+        q = _queries(rng, 2, 15, 20, 0.25)
+        for l in range(3):
+            _sparse(out, f"odd/pyr{l}", _rows(q))
+        _sparse(out, "odd/lookup", _positions(q))
+    elif name.startswith("trace_"):
+        H, W, _, n_lookup, _ = (int(v) for v in out["meta"])
+        ev = out.pop("voxel/events")
+        out["voxel/seed"] = np.array(synth.seed_for(9, 2))
+        assert np.array_equal(synth.events(len(ev), H, W, int(out["voxel/seed"])), ev)
+        del out["rec_img0"]                                   # == warp0/in
+        cells = rng.random(out["voxel/grid"].shape) < 0.25
+        _sparse(out, "voxel/grid", cells)
+        _sparse(out, "voxel/normalised", cells)
+        q = _queries(rng, *out["corr/fmap1"].shape[:1], *out["corr/fmap1"].shape[2:], 0.2)
+        _sparse(out, "corr/fmap1", _positions(q))
+        for l in range(4):
+            _sparse(out, f"corr/pyr{l}", _rows(q))
+        for k in range(n_lookup):
+            if f"lookup{k}/out" in out:
+                _sparse(out, f"lookup{k}/out", _positions(q))
+        _warp_boxes(out, H, W, "warp0/in", "warp0/out", ("warp0/flow", "flow_final"), "warp1/in", "warp1/out",
+                    "warp1/flow", channels=4)
+    elif name.startswith("trace3_"):
+        H, W, _, frames, _, _ = (int(v) for v in out["meta"])
+        for f in range(frames):
+            n_lookup = int(out[f"f{f}/counts"][0])
+            ev_t = out.pop(f"f{f}/ev_t")
+            ev = np.stack([ev_t] + [out.pop(f"f{f}/ev_{c}").astype(np.float64) for c in "xyp"], axis=1)
+            out[f"f{f}/seed"] = np.array(synth.seed_for(1, 3 + f))
+            assert np.array_equal(synth.events(len(ev), H, W, int(out[f"f{f}/seed"])), ev)
+            for k in range(n_lookup - 1):                     # only the last lookup's output is stored
+                del out[f"f{f}/coords{k}"]
+            q = _queries(rng, *out[f"f{f}/fmap1"].shape[:1], *out[f"f{f}/fmap1"].shape[2:], 0.2)
+            _sparse(out, f"f{f}/fmap1", _positions(q))
+            _sparse(out, f"f{f}/lookup_last", _positions(q))
+            _warp_boxes(out, H, W, f"f{f}/warp0_in", f"f{f}/warp0_out", (f"f{f}/flow_final",), f"f{f}/warp1_in",
+                        f"f{f}/warp1_out", None, channels=2)
+    return out
 
 
 # ------------------------------------------------------------------ voxel ---

@@ -56,21 +56,41 @@ def test_tiling_helpers(bench):
     assert rows.shape == (7, 2) and torch.equal(rows[3], rows[0]) and torch.equal(rows[6], rows[0])
 
 
-def test_reference_arm_prints_the_same_config_and_honours_steps(bench):
+def test_reference_arm_prints_the_same_config_and_honours_steps(bench, tmp_path):
     env = dict(os.environ, PYTHONDONTWRITEBYTECODE="1")
-    res = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--steps", "1", "--warmup", "3"],
-                         capture_output=True, text=True, timeout=600, env=env, cwd=ROOT)
+    res = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--steps", "1", "--warmup", "3",
+                          "--dump-outputs", str(tmp_path)], capture_output=True, text=True, timeout=600, env=env, cwd=ROOT)
     assert res.returncode == 0, res.stderr
     line = json.loads(res.stdout.strip().splitlines()[-1])
     assert line["impl"] == "reference" and line["steps"] == 1 and line["warmup"] == 3 and line["scaling"] == "strong"
     assert line["config"] == bench.public_config(bench.make_cfg("configs[4]"), 1)
     assert line["cpu_baseline"]["kind"] == "port" and line["e2e"]["h2d_bytes_per_step"] == 0 and line["gpu_launches"] == 0
     assert line["value"] > 0 and line["unit"] == "frames/s"
+    names = sorted(os.listdir(tmp_path))
+    assert names == sorted(["voxel.npy", "warped_frame.npy", "warped_codes.npy"] + [f"lookup{k}.npy" for k in range(6)])
+    assert all(np.load(tmp_path / n).dtype == np.float32 for n in names)
     # under torchrun only rank 0 runs the CPU arm; the other ranks exit 0 without a line
     env2 = dict(env, RANK="1", WORLD_SIZE="2", LOCAL_RANK="1")
     res2 = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--gpus", "2", "--steps", "1"],
                           capture_output=True, text=True, timeout=120, env=env2, cwd=ROOT)
     assert res2.returncode == 0 and res2.stdout.strip() == ""
+
+
+def test_dump_outputs_is_a_fixed_bounded_sample(bench, tmp_path):
+    big = torch.arange(3 * 10 ** 6, dtype=torch.float32).reshape(3, 10 ** 6)
+    outs = [torch.full((2, 3), float(k)) for k in range(6)]
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), [np.ones((2, 2), np.float32)] * 2, outs, big, big + 1)
+    names = sorted(os.listdir(tmp_path / "a"))
+    assert len(names) == 9 and sum(os.path.getsize(tmp_path / "a" / n) for n in names) <= 64 << 20
+    for n in names:
+        a = np.load(tmp_path / "a" / n)
+        assert a.dtype == np.float32 and np.array_equal(a, np.load(tmp_path / "b" / n))
+    assert np.array_equal(np.load(tmp_path / "a" / "lookup3.npy"), np.full(6, 3.0, np.float32))     # small: whole
+    assert np.array_equal(np.load(tmp_path / "a" / "voxel.npy"), np.ones(8, np.float32))
+    frame = np.load(tmp_path / "a" / "warped_frame.npy")                                            # large: sampled
+    assert 0 < frame.size < big.numel() and np.all(np.diff(frame) >= 0)
+    assert np.array_equal(np.load(tmp_path / "a" / "warped_codes.npy"), frame + 1)                 # same positions
 
 
 def test_stock_torch_comparator_restates_the_reference_ops():

@@ -16,8 +16,9 @@ reference checkout, SURVEY F4) are run twice on the same synthetic event stream:
 
 PSNR is loss.py:15-24's formula against a fixed synthetic ground-truth sequence; the gate is |dPSNR| <= 0.01 dB per
 frame for BOTH model modes, and the perturbed reconstruction itself must sit >= 50 dB from the stock one.
-This needs /root/reference (build container only): skipped on the GPU box, where tests/test_gpu_parity*.py replay the
-recorded multi-frame traces through the real kernels instead.
+This runs the original project's networks, which are not part of this repository: set CISTA_REFERENCE to a checkout of
+it; without one the test is skipped, and tests/test_gpu_parity*.py replay the recorded multi-frame traces through the
+real kernels instead.
 """
 import argparse
 import math
@@ -29,8 +30,8 @@ import numpy as np
 import pytest
 import torch
 
-REF = os.environ.get("CISTA_REFERENCE", "/root/reference")
-pytestmark = pytest.mark.skipif(not os.path.isdir(REF), reason="reference checkout not present (GPU box)")
+REF = os.environ.get("CISTA_REFERENCE", "")
+pytestmark = pytest.mark.skipif(not os.path.isdir(REF), reason="CISTA_REFERENCE does not name a checkout of the original project")
 
 H, W, NEV, FRAMES = 180, 240, 15000, 10
 

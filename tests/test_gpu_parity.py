@@ -595,10 +595,10 @@ def test_corr_golden(golden, cuda_device, precision, tol):
     assert len(blk.corr_pyramid) == 4
     for l in range(4):
         assert tuple(blk.corr_pyramid[l].shape) == g[f"pyr{l}"].shape
-        assert corr_err(blk.corr_pyramid[l].cpu().numpy(), g[f"pyr{l}"]) <= tol, f"level {l}"
+        assert corr_err(*g.pick(f"pyr{l}", blk.corr_pyramid[l].cpu().numpy())) <= tol, f"level {l}"
     out = blk(dev_t(g["coords"], cuda_device))
     assert tuple(out.shape) == g["lookup"].shape and out.is_contiguous()
-    assert corr_err(out.cpu().numpy(), g["lookup"]) <= tol
+    assert corr_err(*g.pick("lookup", out.cpu().numpy())) <= tol
     vol = cf.CorrBlock.corr(dev_t(g["fmap1"], cuda_device), dev_t(g["fmap2"], cuda_device), precision=precision)
     assert tuple(vol.shape) == (1, 16, 24, 1, 16, 24)
 
@@ -662,12 +662,12 @@ def test_corr_golden_odd_sizes(golden, cuda_device):
                        precision="fp32")
     for l in range(3):
         assert tuple(blk.corr_pyramid[l].shape) == g[f"odd/pyr{l}"].shape
-        assert corr_err(blk.corr_pyramid[l].cpu().numpy(), g[f"odd/pyr{l}"]) <= 1e-5
-    assert corr_err(blk(dev_t(g["odd/coords"], cuda_device)).cpu().numpy(), g["odd/lookup"]) <= 1e-5
+        assert corr_err(*g.pick(f"odd/pyr{l}", blk.corr_pyramid[l].cpu().numpy())) <= 1e-5
+    assert corr_err(*g.pick("odd/lookup", blk(dev_t(g["odd/coords"], cuda_device)).cpu().numpy())) <= 1e-5
     blk_tc = cf.CorrBlock(dev_t(g["odd/fmap1"], cuda_device), dev_t(g["odd/fmap2"], cuda_device), num_levels=3, radius=3,
                           precision="tf32")  # 15x20: N % 4 == 0, odd h -> un-fused tensor-core path
     for l in range(3):
-        assert corr_err(blk_tc.corr_pyramid[l].cpu().numpy(), g[f"odd/pyr{l}"]) <= 1e-3
+        assert corr_err(*g.pick(f"odd/pyr{l}", blk_tc.corr_pyramid[l].cpu().numpy())) <= 1e-3
 
 
 @pytest.mark.parametrize("h,w,levels,radius", [(16, 24, 4, 4), (15, 20, 3, 3)])
@@ -699,11 +699,12 @@ def test_corr_block_backward_matches_autograd_of_the_reference_ops(cuda_device, 
 
 
 def test_lookup_on_reference_pyramid(golden, cuda_device):
-    """Feed the REFERENCE's pyramid to our lookup: isolates the gather from the GEMM."""
+    """Feed the REFERENCE's pyramid to our lookup: isolates the gather from the GEMM.  (The fixture stores the pyramid
+    rows of a sample of the queries; a query's lookup reads only its own rows.)"""
     g = golden("corr")
     pyr = [dev_t(g[f"pyr{l}"], cuda_device) for l in range(4)]
     out = cf.corr_lookup(pyr, dev_t(g["coords"], cuda_device), 4)
-    assert corr_err(out.cpu().numpy(), g["lookup"]) <= 1e-4
+    assert corr_err(*g.pick("lookup", out.cpu().numpy())) <= 1e-4
     assert np.abs(out.cpu().numpy()[0, :, 0, 0]).max() == 0.0  # query far outside: zero padding everywhere
 
 
@@ -749,24 +750,25 @@ def test_model_trace_replay(golden, cuda_device, trace):
     replayed through the CUDA path (real feature / flow statistics, ImagePadder shapes)."""
     g = golden(trace)
     H, W, nev, n_lookup, n_warp = (int(v) for v in g["meta"])
-    grid = cf.events_to_voxel_grid(g["voxel/events"], 5, W, H, mode="deterministic")
-    assert np.array_equal(bits(grid), bits(g["voxel/grid"]))
-    np.testing.assert_allclose(cf.event_preprocess(grid, "std", True), g["voxel/normalised"], rtol=1e-5, atol=1e-5)
+    grid = cf.events_to_voxel_grid(synth.events(nev, H, W, int(g["voxel/seed"])), 5, W, H, mode="deterministic")
+    got, ref = g.pick("voxel/grid", grid)
+    assert np.array_equal(bits(got), bits(ref))
+    np.testing.assert_allclose(*g.pick("voxel/normalised", cf.event_preprocess(grid, "std", True)), rtol=1e-5, atol=1e-5)
     blk = cf.CorrBlock(dev_t(g["corr/fmap1"], cuda_device), dev_t(g["corr/fmap2"], cuda_device), num_levels=4, radius=4)
     for l in range(4):
-        assert corr_err(blk.corr_pyramid[l].cpu().numpy(), g[f"corr/pyr{l}"]) <= 1e-3
+        assert corr_err(*g.pick(f"corr/pyr{l}", blk.corr_pyramid[l].cpu().numpy())) <= 1e-3
     for k in range(n_lookup):
         if f"lookup{k}/out" in g:
             out = blk(dev_t(g[f"lookup{k}/coords"], cuda_device))
-            assert corr_err(out.cpu().numpy(), g[f"lookup{k}/out"]) <= 1e-3
+            assert corr_err(*g.pick(f"lookup{k}/out", out.cpu().numpy())) <= 1e-3
     frame = cf.FrameWarp("forward")
     for k in range(n_warp):
         out = frame.warp_frame(dev_t(g[f"warp{k}/in"], cuda_device), dev_t(g[f"warp{k}/flow"], cuda_device))
-        np.testing.assert_allclose(out.cpu().numpy(), g[f"warp{k}/out"], rtol=0, atol=1e-4)
+        np.testing.assert_allclose(*g.pick(f"warp{k}/out", out.cpu().numpy()), rtol=0, atol=1e-4)
     wi, wz = cf.warp_frame_and_codes(dev_t(g["warp0/in"], cuda_device), dev_t(g["warp1/in"], cuda_device),
                                      dev_t(g["flow_final"], cuda_device), "forward")
-    np.testing.assert_allclose(wi.cpu().numpy(), g["warp0/out"], rtol=0, atol=1e-4)
-    np.testing.assert_allclose(wz.cpu().numpy(), g["warp1/out"], rtol=0, atol=1e-4)
+    np.testing.assert_allclose(*g.pick("warp0/out", wi.cpu().numpy()), rtol=0, atol=1e-4)
+    np.testing.assert_allclose(*g.pick("warp1/out", wz.cpu().numpy()), rtol=0, atol=1e-4)
 
 
 # ------------------------------------------------- agreement summaries (run last) ---

@@ -226,13 +226,16 @@ def test_sharding_world_size_2_gloo(tmp_path):
     assert "OK 0" in res.stdout and "OK 1" in res.stdout
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/e2v"), reason="reference checkout only exists in the build container")
+REF = os.environ.get("CISTA_REFERENCE", "")
+
+
+@pytest.mark.skipif(not os.path.isdir(os.path.join(REF, "e2v")), reason="CISTA_REFERENCE does not name a checkout of the original project")
 def test_install_against_the_real_reference_modules():
     """install() rebinds the names inside the reference's own modules (CPU: import + rebind only)."""
     code = r"""
 import sys, types
 sys.dont_write_bytecode = True
-sys.path.insert(0, "/root/reference"); sys.path.insert(0, %r)
+sys.path.insert(0, %r); sys.path.insert(0, %r)
 mpl = types.ModuleType("matplotlib"); plt = types.ModuleType("matplotlib.pyplot"); mpl.pyplot = plt
 sys.modules["matplotlib"] = mpl; sys.modules["matplotlib.pyplot"] = plt
 oc = types.ModuleType("omegaconf")
@@ -256,7 +259,7 @@ assert isinstance(m.frame_warp, cf.FrameWarp)       # the model now owns OUR Fra
 cf.uninstall()
 assert e2v.e2v_model.FrameWarp is not cf.FrameWarp
 print("OK", len(done))
-""" % ROOT
+""" % (REF, ROOT)
     res = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, timeout=600)
     assert res.returncode == 0 and "OK" in res.stdout, res.stdout + res.stderr
 

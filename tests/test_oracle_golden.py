@@ -10,6 +10,7 @@ import numpy as np
 import pytest
 import torch
 
+from cistaflow_b200 import synth
 from oracle import explicit, ref_port
 
 VOXEL_CASES = ["base", "dense_hot", "single", "two_same_t", "empty"]
@@ -97,16 +98,17 @@ def test_corr_pyramid_and_lookup(golden, prefix, levels, radius):
     f1, f2, coords = g[prefix + "fmap1"], g[prefix + "fmap2"], g[prefix + "coords"]
     pyr = ref_port.corr_pyramid(torch.from_numpy(f1), torch.from_numpy(f2), levels)
     for l in range(levels):
-        assert np.array_equal(pyr[l].numpy(), g[f"{prefix}pyr{l}"])
+        assert np.array_equal(*g.pick(f"{prefix}pyr{l}", pyr[l].numpy()))
     out = ref_port.corr_lookup(pyr, torch.from_numpy(coords), radius)
-    assert np.array_equal(out.numpy(), g[prefix + "lookup"])
+    assert np.array_equal(*g.pick(prefix + "lookup", out.numpy()))
     # explicit: fp64 contraction rounded once, explicit pooling + transposed window
     ex = explicit.corr_pyramid(f1, f2, levels)
     for l in range(levels):
         assert ex[l].shape == g[f"{prefix}pyr{l}"].shape
-        np.testing.assert_allclose(ex[l], g[f"{prefix}pyr{l}"], rtol=0, atol=2e-5)
+        np.testing.assert_allclose(*g.pick(f"{prefix}pyr{l}", ex[l]), rtol=0, atol=2e-5)
+    # (a sampled query's lookup reads only its own, stored, pyramid rows)
     ex_out = explicit.corr_lookup([g[f"{prefix}pyr{l}"] for l in range(levels)], coords, radius)
-    np.testing.assert_allclose(ex_out, g[prefix + "lookup"], rtol=0, atol=2e-5)
+    np.testing.assert_allclose(*g.pick(prefix + "lookup", ex_out), rtol=0, atol=2e-5)
 
 
 def test_lookup_window_is_transposed(golden):
@@ -117,8 +119,8 @@ def test_lookup_window_is_transposed(golden):
     good = explicit.corr_lookup(pyr, coords, 4)
     k = 9
     swapped = good.reshape(1, 4, k, k, 16, 24).transpose(0, 1, 3, 2, 4, 5).reshape(good.shape)
-    assert np.abs(good - g["lookup"]).max() < 2e-5
-    assert np.abs(swapped - g["lookup"]).max() > 0.1
+    assert np.abs(np.subtract(*g.pick("lookup", good))).max() < 2e-5
+    assert np.abs(np.subtract(*g.pick("lookup", swapped))).max() > 0.1
 
 
 @pytest.mark.parametrize("trace", ["trace_eiflow", "trace_eraft"])
@@ -126,23 +128,23 @@ def test_model_trace_replay_through_oracle(golden, trace):
     """Hot-path calls recorded inside the reference models replay through the oracle."""
     g = golden(trace)
     H, W, nev, n_lookup, n_warp = (int(v) for v in g["meta"])
-    grid = ref_port.voxel_grid_numpy(g["voxel/events"], 5, W, H)
-    assert np.array_equal(grid, g["voxel/grid"])
-    np.testing.assert_allclose(ref_port.preprocess_numpy(grid, "std", True), g["voxel/normalised"], rtol=0, atol=1e-6)
+    grid = ref_port.voxel_grid_numpy(synth.events(nev, H, W, int(g["voxel/seed"])), 5, W, H)
+    assert np.array_equal(*g.pick("voxel/grid", grid))
+    np.testing.assert_allclose(*g.pick("voxel/normalised", ref_port.preprocess_numpy(grid, "std", True)), rtol=0, atol=1e-6)
     pyr = ref_port.corr_pyramid(torch.from_numpy(g["corr/fmap1"]), torch.from_numpy(g["corr/fmap2"]), 4)
     for l in range(4):
-        assert np.array_equal(pyr[l].numpy(), g[f"corr/pyr{l}"])
+        assert np.array_equal(*g.pick(f"corr/pyr{l}", pyr[l].numpy()))
     for k in range(n_lookup):
         if f"lookup{k}/out" in g:
             out = ref_port.corr_lookup(pyr, torch.from_numpy(g[f"lookup{k}/coords"]), 4)
-            assert np.array_equal(out.numpy(), g[f"lookup{k}/out"])
+            assert np.array_equal(*g.pick(f"lookup{k}/out", out.numpy()))
     assert n_warp == 2
     for k in range(n_warp):
         out = ref_port.warp(torch.from_numpy(g[f"warp{k}/in"]), torch.from_numpy(g[f"warp{k}/flow"]), "forward")
-        assert np.array_equal(out.numpy(), g[f"warp{k}/out"])
+        assert np.array_equal(*g.pick(f"warp{k}/out", out.numpy()))
     # the codes were warped with the x0.5 down-sampled flow (e2v/e2v_model.py:190)
     half = ref_port.downsample_flow(torch.from_numpy(g["flow_final"]))
-    assert np.array_equal(half.numpy(), g["warp1/flow"])
+    assert np.array_equal(*g.pick("warp1/flow", half.numpy()))
 
 
 MVSEC_CASES = ["base", "binary", "dense", "two"]
@@ -190,8 +192,8 @@ def test_fwl_ref_port_bit_exact(golden):
 
 
 def trace3_events(g, f):
-    return np.stack([g[f"f{f}/ev_t"], g[f"f{f}/ev_x"].astype(np.float64), g[f"f{f}/ev_y"].astype(np.float64),
-                     g[f"f{f}/ev_p"].astype(np.float64)], axis=1)
+    H, W, nev = (int(v) for v in g["meta"][:3])
+    return synth.events(nev, H, W, int(g[f"f{f}/seed"]))
 
 
 @pytest.mark.parametrize("trace", ["trace3_eiflow", "trace3_eraft"])
@@ -207,12 +209,12 @@ def test_multi_frame_trace_through_oracle(golden, trace):
         out = ref_port.corr_lookup(pyr, torch.from_numpy(g[f"f{f}/coords{n_lookup - 1}"]), 4)
         # (the stored lookups came from a CorrBlock built inside the running model: same calls, but the sgemm blocking of
         #  a D = 32 product differs between the two contexts -- 1e-7 relative, not bit-exact)
-        ref = g[f"f{f}/lookup_last"]
-        assert np.abs(out[:, ::4].numpy() - ref).max() <= 1e-6 * np.abs(ref).max()
+        got, ref = g.pick(f"f{f}/lookup_last", out[:, ::4].numpy())
+        assert np.abs(got - ref).max() <= 1e-6 * np.abs(ref).max()
         flow = torch.from_numpy(g[f"f{f}/flow_final"])
         wi, wz = ref_port.warp_frame_and_codes(torch.from_numpy(g[f"f{f}/warp0_in"]), torch.from_numpy(g[f"f{f}/warp1_in"]),
                                                flow, "forward")
-        assert np.array_equal(wi.numpy(), g[f"f{f}/warp0_out"]) and np.array_equal(wz.numpy(), g[f"f{f}/warp1_out"])
+        assert np.array_equal(*g.pick(f"f{f}/warp0_out", wi.numpy())) and np.array_equal(*g.pick(f"f{f}/warp1_out", wz.numpy()))
         ev = trace3_events(g, f)
         assert ev.shape == (nev, 4) and np.all(np.diff(ev[:, 0]) >= 0)
     # the recurrence is live: consecutive frames warp different states with different flows
