@@ -22,8 +22,11 @@ from . import _lib
 # "auto" (default): tensor cores, operands carrying an 11-bit significand either way -- TF32 words rounded by the TMA, or
 # fp16 copies scaled per batch item where that measured faster (wide maps); the two agree to fp32 summation-order noise
 # and the end-to-end PSNR gate (tests/test_e2e_psnr.py) is taken with exactly this operand rounding.
+# "3xtf32": tensor cores with each operand split into two TF32 terms (three MMAs per K step): the fp32 accuracy of the
+# reference's matmul (held to the same 1e-5 as "fp32"), on the tensor cores instead of the SIMT kernel.
 DEFAULT_PRECISION = os.environ.get("CISTAFLOW_CORR_PRECISION", "auto")
-_PREC = {"tf32": _lib.CORR_TF32, "fp32": _lib.CORR_FP32, "f16": _lib.CORR_F16, "auto": _lib.CORR_AUTO}
+_PREC = {"tf32": _lib.CORR_TF32, "fp32": _lib.CORR_FP32, "f16": _lib.CORR_F16, "auto": _lib.CORR_AUTO,
+         "3xtf32": _lib.CORR_3XTF32}
 
 
 def coords_grid(batch, ht, wd, device=None):
@@ -44,7 +47,7 @@ def build_pyramid(fmap1: torch.Tensor, fmap2: torch.Tensor, num_levels: int = 4,
     B, D, h, w = fmap1.shape
     prec = precision or DEFAULT_PRECISION
     lib = _lib.load()
-    if prec in ("tf32", "f16", "auto") and (D % 32 != 0 or (h * w) % 4 != 0):
+    if prec in ("tf32", "f16", "auto", "3xtf32") and (D % 32 != 0 or (h * w) % 4 != 0):
         prec = "fp32"  # shapes the tensor-core tiling does not cover (never the model's: D=256, h,w % 4 == 0)
     dev = fmap1.device
     shapes = [(B * h * w, 1, h >> l, w >> l) for l in range(num_levels)]

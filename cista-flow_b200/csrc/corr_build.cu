@@ -25,6 +25,7 @@ int corr_volume_tensor_core(const float *f1, const float *f2, int B, int D, int 
                             size_t ws_bytes, int flags, int *fused_levels, cudaStream_t stream);
 bool corr_tensor_core_supported(int D, int h, int w);
 size_t corr_tc_workspace_bytes(int B, int D, int h, int w);
+size_t corr_x3_workspace_bytes(int B, int D, int h, int w);
 
 // CF_TC_FLAGS (debug / experiments only, see corr_build_tc.cu)
 static int tc_flags() {
@@ -141,7 +142,9 @@ avg_pool_two_levels_kernel(const float *__restrict__ in, float *__restrict__ out
 }  // namespace cf
 
 extern "C" size_t cf_corr_workspace_bytes(int B, int D, int h, int w, int, int precision) {
-    if ((precision != CF_CORR_F16 && precision != CF_CORR_AUTO) || B <= 0 || D <= 0 || h <= 0 || w <= 0) return 0;
+    if (B <= 0 || D <= 0 || h <= 0 || w <= 0) return 0;
+    if (precision == CF_CORR_3XTF32) return cf::corr_x3_workspace_bytes(B, D, h, w);
+    if (precision != CF_CORR_F16 && precision != CF_CORR_AUTO) return 0;
     return cf::corr_tc_workspace_bytes(B, D, h, w);
 }
 

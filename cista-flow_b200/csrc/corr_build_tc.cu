@@ -186,6 +186,13 @@ __device__ __forceinline__ void tma_load_3d(void *dst, const CUtensorMap *m, int
         : "memory");
 }
 
+__device__ __forceinline__ void tma_load_4d(void *dst, const CUtensorMap *m, int c0, int c1, int c2, int c3, uint64_t *bar) {
+    asm volatile(
+        "cp.async.bulk.tensor.4d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5, %6}], [%2];"
+        ::"r"(smem_u32(dst)), "l"(reinterpret_cast<uint64_t>(m)), "r"(smem_u32(bar)), "r"(c0), "r"(c1), "r"(c2), "r"(c3)
+        : "memory");
+}
+
 // cta_group::2 variants: the box lands in THIS CTA's shared memory, its bytes complete on the mbarrier at the
 // shared::cluster address `bar_addr` -- the pair leader's `full` barrier (mapa_rank0) for both CTAs of the pair
 __device__ __forceinline__ void tma_load_2d_2sm(void *dst, const CUtensorMap *m, int c0, int c1, uint32_t bar_addr) {
@@ -445,17 +452,24 @@ __device__ __forceinline__ void store_row_chunk(float *dst, const uint32_t (&v)[
 // commits arrive on `empty` / `tfull` of both CTAs; both epilogues arrive on the leader's `tempty`.
 // (A first pair variant only multicast the fmap2 tile to two independent cta_group::1 MMAs: L2 traffic -33 %,
 //  time unchanged -- L2 bandwidth was not the bound.)
-// F16: the operands are fp16 copies of the feature maps (same 11-bit significand as TF32, scaled per batch item by a
+// OM_F16: the operands are fp16 copies of the feature maps (same 11-bit significand as TF32, scaled per batch item by a
 // power of two so that any finite input fits; made by fmap_to_half_kernel).  kind::f16 covers K = 16 per MMA where
 // kind::tf32 covers 8 at the same ~1 accumulator column per clock, and every stage moves half the bytes: the GEMM
 // stops being MMA / load-latency bound and runs at the HBM write rate of the volume.
-template <int CL, bool F16, int ES, int BKT>
+// OM_3XTF32: each operand is split x = hi + lo into two exact TF32 values (fmap_split_tf32_kernel, workspace) and every
+// K = 8 step issues lo.hi + hi.lo + hi.hi into the same accumulator: within ~2^-22 of the exact products, fp32-level
+// accuracy at three times the MMA work.  A stage holds both slices of every 32-column atom side by side
+// ([atom][hi, lo][K rows][32 cols], one 4-D TMA box per operand), so the UMMA descriptors see LBO = two boxes and
+// address the lo slice one box behind the hi slice.  Only the producer and the MMA issuer differ; the epilogue is the TF32 one.
+enum OperandMode { OM_TF32 = 0, OM_F16 = 1, OM_3XTF32 = 2 };
+template <int CL, int OM, int ES, int BKT>
 __global__ void __launch_bounds__(threads(ES), 1)
 corr_tc_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__ CUtensorMap tmap_b,
                const __grid_constant__ CUtensorMap tmap_c, const Params p) {
     extern __shared__ uint8_t smem_raw[];
     uint8_t *smem = reinterpret_cast<uint8_t *>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
-    static_assert(!(F16 && CL == 2), "the CTA-pair variant is tf32 only");
+    constexpr bool F16 = OM == OM_F16, X3 = OM == OM_3XTF32;
+    static_assert(OM == OM_TF32 || CL == 1, "the CTA-pair variant is tf32 only");
     constexpr int EPI_SPLIT = ES, EPI_WARPS = 4 * ES, EPI_BYTES = epi_bytes(ES);
 #ifdef CF_SWAP_SERVICE_WARPS   // experiment: which warp scheduler (warp % 4) hosts the producer / the MMA issuer
     constexpr int PRODUCER_WARP = EPI_WARPS + 1, MMA_WARP = EPI_WARPS;
@@ -465,7 +479,8 @@ corr_tc_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant
     constexpr int BC = F16 ? 64 : 32;                   // operand columns per TMA box (128 bytes)
     constexpr int BKK = F16 ? BK_F16 : BKT;             // K rows per stage (TF32: 64, or 32 for D % 64 != 0 and the CTA-pair kernel)
     constexpr int BOXB = 128 * BKK;                     // bytes of one TMA box: 128-byte rows x BKK
-    constexpr int ABYTES = (BM / BC) * BOXB;            // fmap1 part of a stage
+    constexpr int PARTS = X3 ? 2 : 1;                   // slices per 32-column atom (3xTF32: hi, lo)
+    constexpr int ABYTES = PARTS * (BM / BC) * BOXB;    // fmap1 part of a stage
     constexpr int MMAS = F16 ? BKK / 16 : BKK / 8;      // MMAs per stage
     constexpr int KSTEP = F16 ? 2048 : 1024;            // descriptor start-address advance per MMA
     const int STAGES = p.stages, STAGE_BYTES = p.stage_bytes;
@@ -537,7 +552,7 @@ corr_tc_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant
             uint32_t phase = 0;
             // pair kernel: the leader's barrier counts the bytes of BOTH CTAs' boxes
             const uint32_t tx_bytes = (F16 && p.b_sw64) ? (uint32_t)p.stage_bytes
-                                                       : (uint32_t)(CL * (BM / BC + (CL == 2 ? p.b_half : p.n_boxes_b))) * BOXB;
+                                                       : (uint32_t)(CL * PARTS * (BM / BC + (CL == 2 ? p.b_half : p.n_boxes_b))) * BOXB;
             const int jr = CL == 2 ? rank * (p.BN_mma / 2) : 0;  // first fmap2 column of this CTA inside the tile
             int tile_no = 0;
             int tile = tile_of(0), b = 0, mb = 0, nb = 0;
@@ -588,6 +603,22 @@ corr_tc_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant
                         continue;
                     }
                     mbar_expect_tx(&full[stage], tx_bytes);
+                    if (X3) {   // both slices of each atom in one box: {32 cols, K rows, hi/lo, atoms} (per atom when N % 32 != 0)
+                        if (p.atoms3d) {
+                            tma_load_4d(sa, &tmap_a, 0, krow, 0, i0 / BC, &full[stage]);
+                        } else {
+#pragma unroll
+                            for (int a = 0; a < BM / BC; ++a) tma_load_3d(sa + 2 * a * BOXB, &tmap_a, i0 + BC * a, krow, 0, &full[stage]);
+                        }
+                        if (p.b3d) {
+                            tma_load_4d(sb, &tmap_b, 0, krow, 0, j0 / BC, &full[stage]);
+                        } else {
+                            for (int a = 0; a < p.n_boxes_b; ++a) tma_load_3d(sb + 2 * a * BOXB, &tmap_b, j0 + BC * a, krow, 0, &full[stage]);
+                        }
+                        __syncwarp();
+                        if (++stage == STAGES) { stage = 0; phase ^= 1; }
+                        continue;
+                    }
                     if (p.atoms3d) {
                         tma_load_3d(sa, &tmap_a, 0, krow, i0 / BC, &full[stage]);
                     } else {
@@ -622,7 +653,7 @@ corr_tc_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant
             // descriptor high words are constants of the layout; the low word = start address >> 4 | LBO << 16
             const uint32_t desc_hi = F16 ? (uint32_t)((1024u >> 4) | (1u << 14) | (2u << 29))
                                          : (uint32_t)((512u >> 4) | (1u << 14) | (1u << 29));
-            const uint32_t lbo_bits = ((uint32_t)BOXB >> 4) << 16;   // bytes between column atoms = one TMA box
+            const uint32_t lbo_bits = ((uint32_t)(PARTS * BOXB) >> 4) << 16;   // bytes between column atoms = one TMA box per slice
             // fmap2 slice in the 64-byte swizzle (b_sw64): atoms of 32 columns x 64 B rows, 8-row groups 512 B apart, one
             // atom = BKK x 64 B, and a K step of 16 rows is 1024 B
             const bool sw64 = F16 && p.b_sw64;
@@ -658,7 +689,12 @@ corr_tc_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant
                             for (int kk = 0; kk < MMAS; ++kk) {
                                 const uint64_t da = ((uint64_t)desc_hi << 32) | (uint64_t)(a_lo + (uint32_t)(kk * (KSTEP >> 4)));
                                 const uint64_t db = ((uint64_t)desc_hi_b << 32) | (uint64_t)(b_lo + (uint32_t)kk * kstep_b);
-                                if (F16) umma_f16(d_tmem, da, db, idesc, (uint32_t)((kb | kk) != 0));
+                                if (X3) {   // the small cross terms first, hi.hi last; only the tile's first MMA clears
+                                    constexpr uint32_t LO = (uint32_t)BOXB >> 4;   // the lo slice: one box behind the hi slice
+                                    umma_tf32(d_tmem, da + LO, db, idesc, (uint32_t)((kb | kk) != 0));
+                                    umma_tf32(d_tmem, da, db + LO, idesc, 1u);
+                                    umma_tf32(d_tmem, da, db, idesc, 1u);
+                                } else if (F16) umma_f16(d_tmem, da, db, idesc, (uint32_t)((kb | kk) != 0));
                                 else if (CL == 2) umma_tf32_2sm(d_tmem, da, db, idesc, (uint32_t)((kb | kk) != 0));
                                 else umma_tf32(d_tmem, da, db, idesc, (uint32_t)((kb | kk) != 0));
                             }
@@ -1256,6 +1292,37 @@ fmap_to_half_fused_kernel(const float *__restrict__ f1, const float *__restrict_
     }
 }
 
+// ---- 3xTF32 operand split ----------------------------------------------------------------------------------
+// hi = rn_tf32(x) and lo = rn_tf32(x - hi) for both feature maps (x - hi is exact in fp32).  Both are TF32 values exactly,
+// so the tensor maps read them as plain FLOAT32 and the result does not depend on how the TMA or the MMA treats the low
+// 13 mantissa bits.  No scaling: the fp32 range is kept.  n4 = float4 per map.
+__device__ __forceinline__ float rna_tf32(float x) {
+    uint32_t r;
+    asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(r) : "f"(x));
+    return __uint_as_float(r & 0xFFFFE000u);
+}
+__device__ __forceinline__ void split_tf32(float x, float &hi, float &lo) {
+    hi = rna_tf32(x);
+    lo = rna_tf32(x - hi);
+}
+__global__ void __launch_bounds__(256)
+fmap_split_tf32_kernel(const float4 *__restrict__ f1, const float4 *__restrict__ f2, int64_t n4, float4 *__restrict__ hi1,
+                       float4 *__restrict__ lo1, float4 *__restrict__ hi2, float4 *__restrict__ lo2) {
+    const int64_t stride = (int64_t)gridDim.x * blockDim.x;
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < 2 * n4; i += stride) {
+        const bool first = i < n4;
+        const int64_t j = first ? i : i - n4;
+        const float4 v = __ldg((first ? f1 : f2) + j);
+        float4 h, l;
+        split_tf32(v.x, h.x, l.x);
+        split_tf32(v.y, h.y, l.y);
+        split_tf32(v.z, h.z, l.z);
+        split_tf32(v.w, h.w, l.w);
+        (first ? hi1 : hi2)[j] = h;
+        (first ? lo1 : lo2)[j] = l;
+    }
+}
+
 // ---- host side --------------------------------------------------------------------
 typedef CUresult (*EncodeTiledFn)(CUtensorMap *, CUtensorMapDataType, cuuint32_t, void *, const cuuint64_t *,
                                   const cuuint64_t *, const cuuint32_t *, const cuuint32_t *, CUtensorMapInterleave,
@@ -1341,6 +1408,25 @@ static int make_fmap_tmap3_sw64(CUtensorMap *m, const void *base, int B, int D, 
     return CF_OK;
 }
 
+// 3xTF32 operands: the hi copy of a feature map and its lo copy `lo_off` bytes behind it as ONE tensor whose third
+// dimension selects the slice.  box_atoms > 0 (N % 32 == 0): {32 cols, B*D rows, 2 slices, N/32 atoms}, a box {32, rows, 2,
+// box_atoms} lands as [atom][hi, lo][row][32 cols]; box_atoms == 0: {N cols, B*D rows, 2 slices}, one box {32, rows, 2} per atom
+static int make_split_tmap(CUtensorMap *m, const float *hi, size_t lo_off, int B, int D, int N, int box_rows, int box_atoms) {
+    EncodeTiledFn fn = encode_fn();
+    CF_REQUIRE(fn, CF_ERR_CUDA, "cuTensorMapEncodeTiled not available from the driver");
+    const bool atoms = box_atoms > 0;
+    const cuuint32_t rank = atoms ? 4 : 3;
+    cuuint64_t dims[4] = {atoms ? 32u : (cuuint64_t)N, (cuuint64_t)B * D, 2, (cuuint64_t)N / 32};
+    cuuint64_t strides[3] = {(cuuint64_t)N * sizeof(float), (cuuint64_t)lo_off, 128};
+    cuuint32_t box[4] = {32, (cuuint32_t)box_rows, 2, (cuuint32_t)box_atoms};
+    cuuint32_t estr[4] = {1, 1, 1, 1};
+    CUresult r = fn(m, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, rank, const_cast<float *>(hi), dims, strides, box, estr,
+                    CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B_ATOM_32B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
+                    CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+    CF_REQUIRE(r == CUDA_SUCCESS, CF_ERR_CUDA, "cuTensorMapEncodeTiled (split feature map) failed with CUresult %d", (int)r);
+    return CF_OK;
+}
+
 // 3-D map over the level-0 volume [B][N][N], box {32 cols, 32 rows, 1}, 128B swizzle (store side)
 static int make_volume_tmap(CUtensorMap *m, float *base, int B, int N) {
     EncodeTiledFn fn = encode_fn();
@@ -1367,19 +1453,21 @@ size_t corr_tc_workspace_bytes(int B, int D, int h, int w) {
     return 2 * per_map + align_up((size_t)6 * B * sizeof(float), 256);   // maxima, inverse scales, arrival counters
 }
 
+// 3xTF32: hi and lo copies of both feature maps, [hi1 | lo1 | hi2 | lo2], each B*D*h*w floats rounded up to 256 bytes
+size_t corr_x3_workspace_bytes(int B, int D, int h, int w) {
+    return 4 * align_up((size_t)B * D * h * w * sizeof(float), 256);
+}
+
 // flags (debug/experiments, env CF_TC_FLAGS): bit1 = encode the tensor maps as plain FLOAT32 (operands are
 // then truncated, not rounded, to TF32), bit2 = never fuse the pooling, bit3 = fuse level 1 only, bit4 = per-atom 2-D TMA boxes even when N % 32 == 0.
 int corr_volume_tensor_core(const float *f1, const float *f2, int B, int D, int h, int w, float scale, float *level0,
                             float *level1, float *level2, float *level3, int precision, void *ws, size_t ws_bytes, int flags,
                             int *fused_levels, cudaStream_t stream) {
     using namespace tc;
-    CF_REQUIRE(precision == CF_CORR_TF32 || precision == CF_CORR_F16 || precision == CF_CORR_AUTO, CF_ERR_UNSUPPORTED,
-               "cf_corr_build: CF_CORR_3XTF32 is not implemented yet");
+    CF_REQUIRE(precision == CF_CORR_TF32 || precision == CF_CORR_F16 || precision == CF_CORR_AUTO || precision == CF_CORR_3XTF32,
+               CF_ERR_UNSUPPORTED, "cf_corr_build: precision %d has no tensor-core path", precision);
     CF_REQUIRE(aligned16(f1) && aligned16(f2) && aligned16(level0), CF_ERR_ALIGN, "cf_corr_build: tensors must be 16-byte aligned");
     const int N = h * w;
-    // AUTO resolves to TF32: the fp16-operand variant halves the MMA time and the operand bytes and agrees with
-    // TF32 to summation-order noise (same 11-bit operand significands), but measured NO faster on the B200
-    // (8 x 60x80: GEMM 283 against 277 us, plus 32 us of conversion) -- the kernel is bound on the volume's write side
     // AUTO (round 2): fp16 operands where they measured faster on the B200 -- wide maps whose N is a whole number of
     // 64-column fp16 boxes and enough tiles to amortise the conversion pass (8 x 60x80: 288 against 319 us, 64 x 60x80: 2375
     // against 2580 us) -- TF32 elsewhere (64 x 24x32: 61 against 108 us, 64 x 36x44: 336 against 374, 1 x 80x124: 183 against 205)
@@ -1387,10 +1475,28 @@ int corr_volume_tensor_core(const float *f1, const float *f2, int B, int D, int 
         precision = (N % 64 == 0 && N >= 2048 && (int64_t)B * N >= 19200 && D % BK_F16 == 0 && ws != nullptr &&
                      ws_bytes >= corr_tc_workspace_bytes(B, D, h, w)) ? CF_CORR_F16 : CF_CORR_TF32;
     if (precision == CF_CORR_F16 && D % BK_F16 != 0) precision = CF_CORR_TF32;   // the fp16 stages hold 128 K rows
-    const bool f16 = precision == CF_CORR_F16;
+    const bool f16 = precision == CF_CORR_F16, x3 = precision == CF_CORR_3XTF32;
     const int BC = f16 ? 64 : 32;   // operand columns per TMA box
     const void *a = f1, *bm = f2;
     const float *inv_scale = nullptr;
+    size_t lo_off = 0;              // 3xTF32: bytes from a hi copy to its lo copy
+    if (x3) {
+        const size_t need = corr_x3_workspace_bytes(B, D, h, w);
+        CF_REQUIRE(ws && ws_bytes >= need, CF_ERR_WORKSPACE, "cf_corr_build: workspace too small for CF_CORR_3XTF32 (%zu < %zu)",
+                   ws_bytes, need);
+        CF_REQUIRE(aligned16(ws), CF_ERR_ALIGN, "cf_corr_build: workspace not 16-byte aligned");
+        lo_off = need / 4;
+        char *base = reinterpret_cast<char *>(ws);
+        float4 *hi1 = reinterpret_cast<float4 *>(base), *lo1 = reinterpret_cast<float4 *>(base + lo_off);
+        float4 *hi2 = reinterpret_cast<float4 *>(base + 2 * lo_off), *lo2 = reinterpret_cast<float4 *>(base + 3 * lo_off);
+        const int64_t n4 = (int64_t)B * D * N / 4;   // N % 4 == 0 (corr_tensor_core_supported)
+        const int64_t blocks = ceil_div(2 * n4, 256);
+        const int64_t cap = 8 * (int64_t)sm_count();
+        fmap_split_tf32_kernel<<<(unsigned)(blocks < cap ? blocks : cap), 256, 0, stream>>>(
+            reinterpret_cast<const float4 *>(f1), reinterpret_cast<const float4 *>(f2), n4, hi1, lo1, hi2, lo2);
+        CF_LAUNCH_CHECK("fmap_split_tf32_kernel");
+        a = hi1; bm = hi2;
+    }
     if (f16) {
         const size_t need = corr_tc_workspace_bytes(B, D, h, w);
         CF_REQUIRE(ws && ws_bytes >= need, CF_ERR_WORKSPACE, "cf_corr_build: workspace too small for CF_CORR_F16 (%zu < %zu)",
@@ -1500,11 +1606,11 @@ int corr_volume_tensor_core(const float *f1, const float *f2, int B, int D, int 
                                        : ((flags & 2) ? CU_TENSOR_MAP_DATA_TYPE_FLOAT32 : CU_TENSOR_MAP_DATA_TYPE_TFLOAT32);
     p.atoms3d = (N % BC == 0) && !(flags & 16);
     p.b3d = p.atoms3d && (p.BN % BC == 0 || p.tiles_n == 1);
-    const bool pair_req = (flags & 64) && !f16;
+    const bool pair_req = (flags & 64) && !f16 && !x3;
     const int bk = f16 ? BK_F16 : ((pair_req || D % BK_TF32 != 0) ? BK : BK_TF32);          // K rows per stage
     const int boxb = 128 * bk;                 // bytes per TMA box
-    const int a_bytes = (BM / BC) * boxb;
-    p.stage_bytes = a_bytes + p.n_boxes_b * boxb;
+    const int a_bytes = (x3 ? 2 : 1) * (BM / BC) * boxb;
+    p.stage_bytes = a_bytes + (x3 ? 2 : 1) * p.n_boxes_b * boxb;
     p.b_sw64 = 0;
     // (the 128-byte-swizzled slice is one 3-D box only when tiles start on 64-column boundaries -- b3d; with 160-column tiles
     //  it took three 2-D boxes per stage)
@@ -1521,9 +1627,12 @@ int corr_volume_tensor_core(const float *f1, const float *f2, int B, int D, int 
     const int es = (f16 && p.deep == 0 && !(flags & 128) && (SMEM_LIMIT - smem_fixed(2)) / p.stage_bytes >= 2) ? 2 : 1;
     p.stages = (SMEM_LIMIT - smem_fixed(es)) / p.stage_bytes;
     if (p.stages > MAX_STAGES) p.stages = MAX_STAGES;
+    // 3xTF32 stages are twice the TF32 ones (72 KB at BN = 160, 96 KB at BN = 256): a ring of two beside the epilogue
+    CF_REQUIRE(!x3 || p.stages >= 2, CF_ERR_UNSUPPORTED, "cf_corr_build: %d-byte operand stages leave room for %d in shared memory",
+               p.stage_bytes, p.stages);
     // pairs of query tiles as one 256-row UMMA across two CTAs: measured slower than one CTA per tile on the B200
     // (8 x 60x80: 359 against 322 us, see the kernel's header), so only on request (flags bit6)
-    const bool pair = (flags & 64) && p.tiles_m >= 2 && !f16;
+    const bool pair = (flags & 64) && p.tiles_m >= 2 && !f16 && !x3;
     p.ablate = (flags >> 8) & 255;
     // level-0 rows through the LSU instead of TMA bulk stores: helps where the operand loads already need many TMA
     // instructions per stage (N % 32 != 0: 64 x 36x44 398 -> 367 us), costs 2-5 % elsewhere (flags bit0: always TMA)
@@ -1600,12 +1709,16 @@ int corr_volume_tensor_core(const float *f1, const float *f2, int B, int D, int 
     }
     const int smem_bytes = p.stages * p.stage_bytes + p.epi_bytes + 1024 + 256;
     CUtensorMap ta, tb, tcm;
-    if (p.atoms3d) {
+    if (x3) {
+        if (int rc = make_split_tmap(&ta, static_cast<const float *>(a), lo_off, B, D, N, bk, p.atoms3d ? BM / 32 : 0)) return rc;
+    } else if (p.atoms3d) {
         if (int rc = make_fmap_tmap3(&ta, a, B, D, N, dt, bk, BM / BC)) return rc;
     } else {
         if (int rc = make_fmap_tmap(&ta, a, B, D, N, dt, bk)) return rc;
     }
-    if (p.b_sw64) {
+    if (x3) {
+        if (int rc = make_split_tmap(&tb, static_cast<const float *>(bm), lo_off, B, D, N, bk, p.b3d ? p.n_boxes_b : 0)) return rc;
+    } else if (p.b_sw64) {
         if (int rc = make_fmap_tmap3_sw64(&tb, bm, B, D, N, bk, p.BN_mma / 32)) return rc;
     } else if (p.b3d) {
         if (int rc = make_fmap_tmap3(&tb, bm, B, D, N, dt, bk, pair ? p.b_half : p.n_boxes_b)) return rc;
@@ -1620,11 +1733,12 @@ int corr_volume_tensor_core(const float *f1, const float *f2, int B, int D, int 
     CF_CUDA(cudaGetDevice(&dev));
     static bool opt_in[64] = {};
     if (!opt_in[dev & 63]) {
-        CF_CUDA(cudaFuncSetAttribute(corr_tc_kernel<1, false, 1, BK_TF32>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_LIMIT));
-        CF_CUDA(cudaFuncSetAttribute(corr_tc_kernel<1, false, 1, BK>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_LIMIT));
-        CF_CUDA(cudaFuncSetAttribute(corr_tc_kernel<2, false, 1, BK>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_LIMIT));
-        CF_CUDA(cudaFuncSetAttribute(corr_tc_kernel<1, true, 1, BK>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_LIMIT));
-        CF_CUDA(cudaFuncSetAttribute(corr_tc_kernel<1, true, 2, BK>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_LIMIT));
+        CF_CUDA(cudaFuncSetAttribute(corr_tc_kernel<1, OM_TF32, 1, BK_TF32>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_LIMIT));
+        CF_CUDA(cudaFuncSetAttribute(corr_tc_kernel<1, OM_TF32, 1, BK>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_LIMIT));
+        CF_CUDA(cudaFuncSetAttribute(corr_tc_kernel<2, OM_TF32, 1, BK>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_LIMIT));
+        CF_CUDA(cudaFuncSetAttribute(corr_tc_kernel<1, OM_F16, 1, BK>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_LIMIT));
+        CF_CUDA(cudaFuncSetAttribute(corr_tc_kernel<1, OM_F16, 2, BK>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_LIMIT));
+        CF_CUDA(cudaFuncSetAttribute(corr_tc_kernel<1, OM_3XTF32, 1, BK>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_LIMIT));
         opt_in[dev & 63] = true;
     }
     const int sms = sm_count();
@@ -1642,19 +1756,24 @@ int corr_volume_tensor_core(const float *f1, const float *f2, int B, int D, int 
         attr[0].val.clusterDim.z = 1;
         cfg.attrs = attr;
         cfg.numAttrs = 1;
-        CF_CUDA(cudaLaunchKernelEx(&cfg, corr_tc_kernel<2, false, 1, BK>, ta, tb, tcm, p));
+        CF_CUDA(cudaLaunchKernelEx(&cfg, corr_tc_kernel<2, OM_TF32, 1, BK>, ta, tb, tcm, p));
         CF_LAUNCH_CHECK("corr_tc_kernel<pair>");
         return CF_OK;
     }
     const int grid = p.total_tiles < sms ? p.total_tiles : sms;
     if (f16) {
-        if (es == 2) corr_tc_kernel<1, true, 2, BK><<<grid, threads(2), smem_bytes, stream>>>(ta, tb, tcm, p);
-        else corr_tc_kernel<1, true, 1, BK><<<grid, threads(1), smem_bytes, stream>>>(ta, tb, tcm, p);
+        if (es == 2) corr_tc_kernel<1, OM_F16, 2, BK><<<grid, threads(2), smem_bytes, stream>>>(ta, tb, tcm, p);
+        else corr_tc_kernel<1, OM_F16, 1, BK><<<grid, threads(1), smem_bytes, stream>>>(ta, tb, tcm, p);
         CF_LAUNCH_CHECK("corr_tc_kernel<f16>");
         return CF_OK;
     }
-    if (bk == BK_TF32) corr_tc_kernel<1, false, 1, BK_TF32><<<grid, threads(1), smem_bytes, stream>>>(ta, tb, tcm, p);
-    else corr_tc_kernel<1, false, 1, BK><<<grid, threads(1), smem_bytes, stream>>>(ta, tb, tcm, p);
+    if (x3) {
+        corr_tc_kernel<1, OM_3XTF32, 1, BK><<<grid, threads(1), smem_bytes, stream>>>(ta, tb, tcm, p);
+        CF_LAUNCH_CHECK("corr_tc_kernel<3xtf32>");
+        return CF_OK;
+    }
+    if (bk == BK_TF32) corr_tc_kernel<1, OM_TF32, 1, BK_TF32><<<grid, threads(1), smem_bytes, stream>>>(ta, tb, tcm, p);
+    else corr_tc_kernel<1, OM_TF32, 1, BK><<<grid, threads(1), smem_bytes, stream>>>(ta, tb, tcm, p);
     CF_LAUNCH_CHECK("corr_tc_kernel");
     return CF_OK;
 }

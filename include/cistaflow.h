@@ -241,11 +241,14 @@ CF_API int cf_voxel_flow_warp(const float *voxel, const float *displacement, int
 typedef enum cf_corr_precision {
     CF_CORR_TF32 = 0, /* tcgen05.mma kind::tf32, fp32 accumulate in TMEM (default)  */
     CF_CORR_FP32 = 1, /* SIMT FFMA, fp32 operands (reference arithmetic)             */
-    CF_CORR_3XTF32 = 2, /* tcgen05, 3-term split: ~fp32 accuracy at 3x the MMA work   */
+    CF_CORR_3XTF32 = 2, /* tcgen05.mma kind::tf32 on split operands (workspace): x = hi + lo, hi = rn_tf32(x),
+                           lo = rn_tf32(x - hi), three MMAs per K step (lo.hi + hi.lo + hi.hi) into one fp32 accumulator.
+                           Within ~2^-22 of the exact products: fp32 accuracy at three times the TF32 MMA work.  Same
+                           shapes as TF32 (CF_ERR_UNSUPPORTED elsewhere).  Workspace: 4 * round_up(B*D*h*w*4, 256) bytes */
     CF_CORR_F16 = 3,    /* tcgen05.mma kind::f16 on fp16 operand COPIES (workspace): same 11-bit significand as a TF32
                            operand, scaled per batch item by a power of two so that every finite input fits; K = 16
-                           per MMA and half the operand bytes.  Within fp32 summation-order noise of TF32; measured no
-                           faster on a B200 (the kernel is bound on the volume's write side), kept as an option */
+                           per MMA and half the operand bytes.  Within fp32 summation-order noise of TF32; faster than
+                           TF32 on wide maps with many tiles, which is where CF_CORR_AUTO selects it */
     CF_CORR_AUTO = 4    /* the library's choice by shape: fp16 operand copies for wide maps (N % 64 == 0, many tiles), else TF32 */
 } cf_corr_precision;
 
