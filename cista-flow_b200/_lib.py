@@ -56,6 +56,12 @@ SYMBOLS = {
     "cf_corr_lookup": (_i, [ctypes.POINTER(_vp), _vp, _i, _i, _i, _i, _i, _vp, _vp]),
     "cf_corr_lookup_backward": (_i, [_vp, ctypes.POINTER(_vp), _vp, _i, _i, _i, _i, _i, ctypes.POINTER(_vp), _vp, _vp]),
 }
+# every symbol include/cistaflow_altcorr.h declares (the on-demand correlation lookup, compiled into the same library)
+ALTCORR_SYMBOLS = {
+    "cf_corr_alt_workspace_bytes": (_sz, [_i, _i, _i, _i, _i, _i]),
+    "cf_corr_alt_prepare": (_i, [_vp, _vp, _i, _i, _i, _i, _i, _i, _vp, _sz, _vp]),
+    "cf_corr_alt_lookup": (_i, [_vp, _vp, _i, _i, _i, _i, _i, _i, _i, _vp, _vp]),
+}
 
 _lock = threading.Lock()
 _lib = None
@@ -66,7 +72,7 @@ class CistaFlowError(RuntimeError):
 
 
 def load() -> ctypes.CDLL:
-    """dlopen the library and bind every symbol of the header (no GPU needed)."""
+    """dlopen the library and bind every symbol of both headers (no GPU needed)."""
     global _lib
     if _lib is not None:
         return _lib
@@ -78,7 +84,7 @@ def load() -> ctypes.CDLL:
                     f"`python cista-flow_b200/build.py` (or __graft_entry__.build()). "
                     f"There is no CPU / PyTorch fallback for the hot path.")
             lib = ctypes.CDLL(LIB_PATH)
-            for name, (res, args) in SYMBOLS.items():
+            for name, (res, args) in {**SYMBOLS, **ALTCORR_SYMBOLS}.items():
                 fn = getattr(lib, name)  # AttributeError if the .so lacks a declared symbol
                 fn.restype, fn.argtypes = res, args
             _lib = lib

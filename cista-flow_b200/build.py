@@ -20,7 +20,8 @@ INCLUDE = os.path.join(ROOT, "include")
 LIB = os.path.join(HERE, "libcistaflow.so")
 STAMP = os.path.join(HERE, ".libcistaflow.stamp")
 
-SOURCES = ["api.cu", "voxel.cu", "voxel_tiled.cu", "voxel_packed.cu", "warp.cu", "warp_tma.cu", "warp_backward.cu", "fwl.cu", "corr_lookup.cu", "corr_lookup_backward.cu", "corr_build.cu", "corr_build_tc.cu"]
+HEADERS = ["cistaflow.h", "cistaflow_altcorr.h"]
+SOURCES = ["api.cu", "voxel.cu", "voxel_tiled.cu", "voxel_packed.cu", "warp.cu", "warp_tma.cu", "warp_backward.cu", "fwl.cu", "corr_lookup.cu", "corr_lookup_backward.cu", "corr_build.cu", "corr_build_tc.cu", "corr_alt.cu"]
 
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a",
@@ -39,7 +40,7 @@ def _nvcc() -> str:
 
 def _fingerprint() -> str:
     h = hashlib.sha256()
-    files = [os.path.join(CSRC, f) for f in sorted(os.listdir(CSRC))] + [os.path.join(INCLUDE, "cistaflow.h")]
+    files = [os.path.join(CSRC, f) for f in sorted(os.listdir(CSRC))] + [os.path.join(INCLUDE, h) for h in HEADERS]
     for f in files:
         h.update(f.encode())
         with open(f, "rb") as fh:

@@ -178,3 +178,58 @@ class CorrBlock:
             with torch.no_grad():
                 vol = build_pyramid(fmap1, fmap2, 1, precision)[0]
         return vol.view(B, h, w, 1, h, w)
+
+
+# AlternateCorrBlock: "tf32" / "f16" / "auto" run on the tensor cores (TF32 operands), "fp32" / "3xtf32" on the fp32
+# SIMT kernel, so that an fp32-accurate request gets fp32 accuracy
+_ALT_PREC = {"tf32": _lib.CORR_TF32, "f16": _lib.CORR_AUTO, "auto": _lib.CORR_AUTO, "fp32": _lib.CORR_FP32,
+             "3xtf32": _lib.CORR_FP32}
+
+
+class AlternateCorrBlock:
+    """Drop-in for ``DCEIFlow/core/corr/raft_corr.py:175-203`` (RAFT's AlternateCorrBlock): the lookup of
+    ``CorrBlock`` without the all-pairs volume.  The block keeps fmap1 and the average-pooled levels of fmap2
+    (``cf_corr_alt_prepare``, O(B*D*h*w) bytes) and every call computes the dot products around each query on the
+    tensor cores (``cf_corr_alt_lookup``).  The output equals ``CorrBlock(fmap1, fmap2, ...)(coords)`` up to fp32
+    summation order and operand rounding.  Inference-only, like the reference's (it calls alt_cuda_corr.forward)."""
+
+    def __init__(self, fmap1, fmap2, num_levels=4, radius=4, precision=None):
+        self.num_levels = num_levels
+        self.radius = radius
+        prec = precision or DEFAULT_PRECISION
+        if prec not in _ALT_PREC:
+            raise ValueError(f"AlternateCorrBlock: precision {prec!r} is not one of {sorted(_ALT_PREC)}")
+        self.precision = _ALT_PREC[prec]
+        self._check_no_grad(fmap1, fmap2)
+        fmap1, fmap2 = _prep(fmap1, "fmap1"), _prep(fmap2, "fmap2")
+        assert fmap1.shape == fmap2.shape and fmap1.dim() == 4
+        self.shape = tuple(fmap1.shape)
+        B, D, h, w = self.shape
+        lib = _lib.load()
+        dev = fmap1.device
+        with torch.cuda.device(dev):
+            nbytes = lib.cf_corr_alt_workspace_bytes(B, D, h, w, num_levels, self.precision)
+            self.state = _lib.workspace(nbytes, dev)
+            rc = lib.cf_corr_alt_prepare(fmap1.data_ptr(), fmap2.data_ptr(), B, D, h, w, num_levels, self.precision,
+                                         _lib.ptr(self.state), nbytes, _lib.stream_ptr(dev))
+        _lib.check(rc, "cf_corr_alt_prepare")
+
+    @staticmethod
+    def _check_no_grad(*tensors):
+        if torch.is_grad_enabled() and any(t.requires_grad for t in tensors):
+            raise RuntimeError("cistaflow_b200 AlternateCorrBlock is inference-only: an input requires grad "
+                               "(run under torch.no_grad(), or use CorrBlock, which is differentiable)")
+
+    def __call__(self, coords):
+        self._check_no_grad(coords)
+        coords = _prep(coords, "coords")
+        B, D, h, w = self.shape
+        assert tuple(coords.shape) == (B, 2, h, w), "coords do not match the feature maps"
+        k = 2 * self.radius + 1
+        out = torch.empty((B, self.num_levels * k * k, h, w), dtype=torch.float32, device=coords.device)
+        lib = _lib.load()
+        with torch.cuda.device(coords.device):
+            rc = lib.cf_corr_alt_lookup(_lib.ptr(self.state), coords.data_ptr(), B, D, h, w, self.num_levels, self.radius,
+                                        self.precision, out.data_ptr(), _lib.stream_ptr(coords.device))
+        _lib.check(rc, "cf_corr_alt_lookup")
+        return out

@@ -52,13 +52,12 @@
 #include <cuda.h>
 #include <cuda_fp16.h>
 
-#include "common.cuh"
+#include "tcgen05.cuh"
 
 namespace cf {
 
 namespace tc {
 
-constexpr int BM = 128;          // queries per tile (UMMA M)
 constexpr int BK = 32;           // K rows per pipeline stage (4 MMAs of K=8)
 // fp16 operands: 64 K rows per stage.  One SM's TMA unit retires a 3-D box instruction of these shapes about every
 // 320 ns WHATEVER its size between 20 and 40 KB (profiles/r02/tma_probe.txt: {64 cols, 32 rows, 5 atoms} and
@@ -84,7 +83,6 @@ constexpr int SMEM_LIMIT = 227 * 1024;
 __host__ __device__ constexpr int epi_bytes(int es) { return 4 * es * 2 /*double buffer*/ * EPI_BUF_BYTES; }   // 32 KB per ES
 __host__ __device__ constexpr int smem_fixed(int es) { return epi_bytes(es) + 1024 /*align slack*/ + 256 /*barriers*/; }
 __host__ __device__ constexpr int threads(int es) { return 32 * (4 * es + 2); }
-constexpr uint32_t SPIN_LIMIT = 1u << 26;  // ~seconds; a stuck pipeline traps instead of hanging the GPU
 
 struct Params {
     int B, D, N, h, w;
@@ -133,256 +131,6 @@ struct Params {
     float *l2;
     float *l3;
 };
-
-// ---- PTX wrappers ---------------------------------------------------------------
-__device__ __forceinline__ uint32_t smem_u32(const void *p) { return (uint32_t)__cvta_generic_to_shared(p); }
-
-__device__ __forceinline__ void mbar_init(uint64_t *bar, uint32_t count) {
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count) : "memory");
-}
-__device__ __forceinline__ void mbar_expect_tx(uint64_t *bar, uint32_t bytes) {
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void mbar_arrive(uint64_t *bar) {
-    asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory");
-}
-__device__ __forceinline__ bool mbar_try_wait(uint64_t *bar, uint32_t parity) {
-    uint32_t ok;
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-        "selp.u32 %0, 1, 0, p;\n\t}"
-        : "=r"(ok)
-        : "r"(smem_u32(bar)), "r"(parity)
-        : "memory");
-    return ok != 0;
-}
-__device__ __forceinline__ void mbar_wait(uint64_t *bar, uint32_t parity) {
-    uint32_t spins = 0;
-    while (!mbar_try_wait(bar, parity)) {
-        if (++spins > SPIN_LIMIT) __trap();
-    }
-}
-__device__ __forceinline__ void fence_barrier_init() { asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory"); }
-__device__ __forceinline__ void tc_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
-__device__ __forceinline__ void tc_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
-
-__device__ __forceinline__ void tma_prefetch_desc(const CUtensorMap *m) {
-    asm volatile("prefetch.tensormap [%0];" ::"l"(reinterpret_cast<uint64_t>(m)) : "memory");
-}
-// (L2 policy hints -- evict_last on these loads, evict_first on the volume stores -- were measured on the B200:
-//  no effect at any shape, so the plain forms are used)
-__device__ __forceinline__ void tma_load_2d(void *dst, const CUtensorMap *m, int c0, int c1, uint64_t *bar) {
-    asm volatile(
-        "cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];"
-        ::"r"(smem_u32(dst)), "l"(reinterpret_cast<uint64_t>(m)), "r"(smem_u32(bar)), "r"(c0), "r"(c1)
-        : "memory");
-}
-
-__device__ __forceinline__ void tma_load_3d(void *dst, const CUtensorMap *m, int c0, int c1, int c2, uint64_t *bar) {
-    asm volatile(
-        "cp.async.bulk.tensor.3d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5}], [%2];"
-        ::"r"(smem_u32(dst)), "l"(reinterpret_cast<uint64_t>(m)), "r"(smem_u32(bar)), "r"(c0), "r"(c1), "r"(c2)
-        : "memory");
-}
-
-__device__ __forceinline__ void tma_load_4d(void *dst, const CUtensorMap *m, int c0, int c1, int c2, int c3, uint64_t *bar) {
-    asm volatile(
-        "cp.async.bulk.tensor.4d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5, %6}], [%2];"
-        ::"r"(smem_u32(dst)), "l"(reinterpret_cast<uint64_t>(m)), "r"(smem_u32(bar)), "r"(c0), "r"(c1), "r"(c2), "r"(c3)
-        : "memory");
-}
-
-// cta_group::2 variants: the box lands in THIS CTA's shared memory, its bytes complete on the mbarrier at the
-// shared::cluster address `bar_addr` -- the pair leader's `full` barrier (mapa_rank0) for both CTAs of the pair
-__device__ __forceinline__ void tma_load_2d_2sm(void *dst, const CUtensorMap *m, int c0, int c1, uint32_t bar_addr) {
-    asm volatile(
-        "cp.async.bulk.tensor.2d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];"
-        ::"r"(smem_u32(dst)), "l"(reinterpret_cast<uint64_t>(m)), "r"(bar_addr), "r"(c0), "r"(c1)
-        : "memory");
-}
-__device__ __forceinline__ void tma_load_3d_2sm(void *dst, const CUtensorMap *m, int c0, int c1, int c2, uint32_t bar_addr) {
-    asm volatile(
-        "cp.async.bulk.tensor.3d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5}], [%2];"
-        ::"r"(smem_u32(dst)), "l"(reinterpret_cast<uint64_t>(m)), "r"(bar_addr), "r"(c0), "r"(c1), "r"(c2)
-        : "memory");
-}
-// shared::cluster address of the same shared-memory object in CTA 0 of the cluster
-__device__ __forceinline__ uint32_t mapa_rank0(const void *p) {
-    uint32_t r;
-    asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(r) : "r"(smem_u32(p)), "r"(0u));
-    return r;
-}
-__device__ __forceinline__ void mbar_arrive_cluster(uint32_t bar_addr) {
-    asm volatile("mbarrier.arrive.release.cluster.shared::cluster.b64 _, [%0];" ::"r"(bar_addr) : "memory");
-}
-__device__ __forceinline__ uint32_t cluster_ctarank() {
-    uint32_t r;
-    asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
-    return r;
-}
-__device__ __forceinline__ void cluster_sync_all() {
-    asm volatile("barrier.cluster.arrive.release.aligned;\n\tbarrier.cluster.wait.acquire.aligned;" ::: "memory");
-}
-
-// smem (32 rows x 128 B, 128B swizzle) -> global box {32 cols, 32 rows, 1} of the [B][N][N] volume
-__device__ __forceinline__ void tma_store_3d(const CUtensorMap *m, const void *src, int c0, int c1, int c2) {
-    asm volatile("cp.async.bulk.tensor.3d.global.shared::cta.bulk_group [%0, {%2, %3, %4}], [%1];"
-                 ::"l"(reinterpret_cast<uint64_t>(m)), "r"(smem_u32(src)), "r"(c0), "r"(c1), "r"(c2)
-                 : "memory");
-}
-// the two epilogue warps of TMEM lane quarter q (64 threads) meet
-__device__ __forceinline__ void quarter_barrier(int q) { asm volatile("bar.sync %0, 64;" ::"r"(q + 1) : "memory"); }
-__device__ __forceinline__ void tma_store_commit() { asm volatile("cp.async.bulk.commit_group;" ::: "memory"); }
-// at most N committed store groups may still be READING their shared-memory source
-template <int N>
-__device__ __forceinline__ void tma_store_wait_read() { asm volatile("cp.async.bulk.wait_group.read %0;" ::"n"(N) : "memory"); }
-__device__ __forceinline__ void tma_store_wait_all() { asm volatile("cp.async.bulk.wait_group 0;" ::: "memory"); }
-__device__ __forceinline__ void fence_async_smem() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
-
-__device__ __forceinline__ void tmem_alloc(uint32_t *slot, uint32_t cols) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(slot)), "r"(cols) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-}
-__device__ __forceinline__ void tmem_dealloc(uint32_t addr, uint32_t cols) {
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(addr), "r"(cols) : "memory");
-}
-__device__ __forceinline__ void umma_commit(uint64_t *bar) {
-    asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(bar)) : "memory");
-}
-// pair kernel: arrive on the mbarrier at this offset in every CTA of `mask` once the pair's MMAs have completed
-__device__ __forceinline__ void umma_commit_2sm(uint64_t *bar, uint16_t mask) {
-    asm volatile("tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;"
-                 ::"r"(smem_u32(bar)), "h"(mask) : "memory");
-}
-__device__ __forceinline__ void tmem_alloc_2sm(uint32_t *slot, uint32_t cols) {
-    asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(slot)), "r"(cols) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
-}
-__device__ __forceinline__ void tmem_dealloc_2sm(uint32_t addr, uint32_t cols) {
-    asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(addr), "r"(cols) : "memory");
-}
-// M = 256 across the CTA pair: each CTA contributes its 128 fmap1 rows and HALF of the fmap2 tile from its own
-// shared memory (same offsets in both CTAs) and receives its 128 x N accumulator rows in its own TMEM
-__device__ __forceinline__ void umma_tf32_2sm(uint32_t d_tmem, uint64_t a_desc, uint64_t b_desc, uint32_t idesc, uint32_t accumulate) {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "setp.ne.b32 p, %4, 0;\n\t"
-        "tcgen05.mma.cta_group::2.kind::tf32 [%0], %1, %2, %3, p;\n\t}"
-        ::"r"(d_tmem), "l"(a_desc), "l"(b_desc), "r"(idesc), "r"(accumulate)
-        : "memory");
-}
-// D[tmem] (+)= A[smem] * B[smem], tf32 operands, fp32 accumulate
-__device__ __forceinline__ void umma_tf32(uint32_t d_tmem, uint64_t a_desc, uint64_t b_desc, uint32_t idesc, uint32_t accumulate) {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "setp.ne.b32 p, %4, 0;\n\t"
-        "tcgen05.mma.cta_group::1.kind::tf32 [%0], %1, %2, %3, p;\n\t}"
-        ::"r"(d_tmem), "l"(a_desc), "l"(b_desc), "r"(idesc), "r"(accumulate)
-        : "memory");
-}
-// 32 lanes x 32 consecutive columns: thread t <- lane (base+t), columns [col, col+32)
-__device__ __forceinline__ void tmem_ld32(uint32_t taddr, uint32_t (&v)[32]) {
-    asm volatile(
-        "tcgen05.ld.sync.aligned.32x32b.x32.b32 "
-        "{%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15,"
-        "%16,%17,%18,%19,%20,%21,%22,%23,%24,%25,%26,%27,%28,%29,%30,%31}, [%32];"
-        : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7]),
-          "=r"(v[8]), "=r"(v[9]), "=r"(v[10]), "=r"(v[11]), "=r"(v[12]), "=r"(v[13]), "=r"(v[14]), "=r"(v[15]),
-          "=r"(v[16]), "=r"(v[17]), "=r"(v[18]), "=r"(v[19]), "=r"(v[20]), "=r"(v[21]), "=r"(v[22]), "=r"(v[23]),
-          "=r"(v[24]), "=r"(v[25]), "=r"(v[26]), "=r"(v[27]), "=r"(v[28]), "=r"(v[29]), "=r"(v[30]), "=r"(v[31])
-        : "r"(taddr)
-        : "memory");
-}
-// 32 lanes x 16 consecutive columns, registers -> TMEM / TMEM -> registers (the level-1 row parked between two tiles)
-__device__ __forceinline__ void tmem_st16(uint32_t taddr, const uint32_t (&v)[16]) {
-    asm volatile(
-        "tcgen05.st.sync.aligned.32x32b.x16.b32 [%0], {%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15,%16};"
-        ::"r"(taddr), "r"(v[0]), "r"(v[1]), "r"(v[2]), "r"(v[3]), "r"(v[4]), "r"(v[5]), "r"(v[6]), "r"(v[7]), "r"(v[8]), "r"(v[9]),
-          "r"(v[10]), "r"(v[11]), "r"(v[12]), "r"(v[13]), "r"(v[14]), "r"(v[15])
-        : "memory");
-    asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory");
-}
-__device__ __forceinline__ void tmem_ld16(uint32_t taddr, uint32_t (&v)[16]) {
-    asm volatile(
-        "tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15}, [%16];"
-        : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7]), "=r"(v[8]), "=r"(v[9]),
-          "=r"(v[10]), "=r"(v[11]), "=r"(v[12]), "=r"(v[13]), "=r"(v[14]), "=r"(v[15])
-        : "r"(taddr)
-        : "memory");
-    asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-}
-// 16 lanes x 32 columns in the 16x256b fragment layout: thread t <- for every 8-column block j: (lane t/4, columns 8j + 2(t%4), +1) in
-// v[4j], v[4j+1] and (lane t/4 + 8, same columns) in v[4j+2], v[4j+3] -- four threads hold one 32-byte run of a row
-__device__ __forceinline__ void tmem_ld_16x256b_x4(uint32_t taddr, uint32_t (&v)[16]) {
-    asm volatile(
-        "tcgen05.ld.sync.aligned.16x256b.x4.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15}, [%16];"
-        : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7]), "=r"(v[8]), "=r"(v[9]),
-          "=r"(v[10]), "=r"(v[11]), "=r"(v[12]), "=r"(v[13]), "=r"(v[14]), "=r"(v[15])
-        : "r"(taddr)
-        : "memory");
-}
-__device__ __forceinline__ void tmem_st8(uint32_t taddr, const uint32_t (&v)[8]) {
-    asm volatile("tcgen05.st.sync.aligned.32x32b.x8.b32 [%0], {%1,%2,%3,%4,%5,%6,%7,%8};"
-                 ::"r"(taddr), "r"(v[0]), "r"(v[1]), "r"(v[2]), "r"(v[3]), "r"(v[4]), "r"(v[5]), "r"(v[6]), "r"(v[7]) : "memory");
-    asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory");
-}
-__device__ __forceinline__ void tmem_ld8(uint32_t taddr, uint32_t (&v)[8]) {
-    asm volatile("tcgen05.ld.sync.aligned.32x32b.x8.b32 {%0,%1,%2,%3,%4,%5,%6,%7}, [%8];"
-                 : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7]) : "r"(taddr) : "memory");
-    asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-}
-// one lane of the (converged) warp
-__device__ __forceinline__ bool elect_one() {
-    uint32_t pred;
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "elect.sync _|p, 0xffffffff;\n\t"
-        "selp.u32 %0, 1, 0, p;\n\t}"
-        : "=r"(pred));
-    return pred != 0;
-}
-__device__ __forceinline__ void tmem_ld_wait() { asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory"); }
-
-// UMMA shared-memory descriptor, MN-major, 128B swizzle with 32B atoms (see file header)
-__device__ __forceinline__ uint64_t make_desc_mn_sw128(uint32_t saddr, uint32_t lbo = 4096u) {
-    uint64_t d = 0;
-    d |= (uint64_t)((saddr & 0x3FFFFu) >> 4);        // start address            bits [0,14)
-    d |= (uint64_t)(lbo >> 4) << 16;                 // leading byte offset (MN) bits [16,30): bytes per TMA box
-    d |= (uint64_t)(512u >> 4) << 32;                // stride byte offset (K)   bits [32,46)
-    d |= (uint64_t)1 << 46;                          // descriptor version (Blackwell)
-    d |= (uint64_t)1 << 61;                          // layout type 1 = SWIZZLE_128B_BASE32B
-    return d;
-}
-// UMMA shared-memory descriptor, MN-major 16-bit operands, plain 128B swizzle: atoms of 64 columns (128 B) x 8 K rows
-// (1024 B); LBO = bytes between 64-column atoms (one TMA box), SBO = bytes between groups of 8 K rows
-__device__ __forceinline__ uint64_t make_desc_mn_f16(uint32_t saddr) {
-    uint64_t d = 0;
-    d |= (uint64_t)((saddr & 0x3FFFFu) >> 4);
-    d |= (uint64_t)(4096u >> 4) << 16;
-    d |= (uint64_t)(1024u >> 4) << 32;
-    d |= (uint64_t)1 << 46;
-    d |= (uint64_t)2 << 61;                          // SWIZZLE_128B
-    return d;
-}
-// D=f32, A=B=f16, both MN-major, M=128, N=n
-__host__ __device__ inline uint32_t make_idesc_f16(int n) {
-    return (1u << 4) | (0u << 7) | (0u << 10) | (1u << 15) | (1u << 16) | ((uint32_t)(n >> 3) << 17) |
-           ((uint32_t)(BM >> 4) << 24);
-}
-__device__ __forceinline__ void umma_f16(uint32_t d_tmem, uint64_t a_desc, uint64_t b_desc, uint32_t idesc, uint32_t accumulate) {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "setp.ne.b32 p, %4, 0;\n\t"
-        "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}"
-        ::"r"(d_tmem), "l"(a_desc), "l"(b_desc), "r"(idesc), "r"(accumulate)
-        : "memory");
-}
-// instruction descriptor: D=f32, A=B=tf32, both MN-major, M=m (128, or 256 across a CTA pair), N=n
-__host__ __device__ inline uint32_t make_idesc_tf32(int n, int m = BM) {
-    return (1u << 4) | (2u << 7) | (2u << 10) | (1u << 15) | (1u << 16) | ((uint32_t)(n >> 3) << 17) |
-           ((uint32_t)(m >> 4) << 24);
-}
 
 // Debug timeline of CTA 0's first tile (clock64 stamps), read back with cf_debug_tc_timeline().
 __device__ unsigned long long g_tc_timeline[32];

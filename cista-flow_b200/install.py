@@ -14,7 +14,7 @@ therefore rebinds the names *in every reference module that imported them*:
                              eventsToVoxel, eventsToVoxelTorch, events_to_voxel_torch, events_to_neg_pos_voxel_torch
                              (part "mvsec": the second voxeliser)
   ERAFT.corr, ERAFT.eraft    CorrBlock
-  DCEIFlow.core.corr.raft_corr, DCEIFlow.DCEIFlow   CorrBlock
+  DCEIFlow.core.corr.raft_corr, DCEIFlow.DCEIFlow   CorrBlock, AlternateCorrBlock
 
 after which ``model_mode`` 'cista-eiflow' / 'cista-eraft' run unchanged on the
 CUDA path.  ``uninstall()`` restores the originals.  The reference checkout must
@@ -33,7 +33,7 @@ _VOXEL = {name: getattr(event_process, name) for name in (
     "events_to_voxel_grid", "events_to_voxel_grid_pol", "events_to_voxel_grid_pytorch",
     "event_preprocess", "event_preprocess_pytorch")}
 _WARP = {name: getattr(flow_utils, name) for name in ("backWarp", "forwardWarp", "FrameWarp")}
-_CORR = {"CorrBlock": corr.CorrBlock}
+_CORR = {"CorrBlock": corr.CorrBlock, "AlternateCorrBlock": corr.AlternateCorrBlock}
 _FWL = {"voxel_warping_flow_loss": loss_mod.voxel_warping_flow_loss}
 _MVSEC = {name: getattr(mvsec_utils, name) for name in (
     "eventsToVoxel", "eventsToVoxelTorch", "events_to_voxel_torch", "events_to_neg_pos_voxel_torch")}
