@@ -11,17 +11,10 @@
 // Two accumulation modes:
 //   ATOMIC         sum order unspecified -> agrees with the reference to <= 1e-5.
 //                  fp32 RED.ADD resolved in L2; the batch is processed in chunks
-//                  of windows whose grids + events fit in L2 (<= 48 MB), each chunk
-//                  running zero -> scatter -> statistics -> normalise-in-place
+//                  of windows whose grids + events fit in L2 (kL2ChunkBytes), each
+//                  chunk running zero -> scatter -> statistics -> normalise-in-place
 //                  back to back, so a grid is read and written in L2 and reaches
 //                  HBM exactly once.
-//                  Measured dead end, kept behind CF_VOXEL_FLAGS=2 for the record:
-//                  privatising the grid in the distributed shared memory of a
-//                  thread-block cluster and scattering with
-//                  red.shared::cluster.add.f32 (voxel_cluster_kernel).  DSMEM
-//                  atomics sustain ~19 G adds/s chip-wide vs ~69 G/s for L2
-//                  atomics on a B200, so that path is 2-4x SLOWER than the L2 one
-//                  (scripts/voxel_microbench.py).
 //   DETERMINISTIC  bit-exact.  The reference accumulates every cell
 //                  sequentially in event order, all bin-ti ("left")
 //                  contributions before all bin-ti+1 ("right") ones (two
@@ -34,30 +27,35 @@
 // (ATOMG instead of RED) give each add's previous value o, and sum f(o + w) - f(o) telescopes to the final
 // grid's sum / sum of squares / non-zero count, so the separate statistics pass disappears.  Correct (all parity
 // tests green) but 1.4-4x SLOWER end to end on the B200 (8x180x240: 24.4 against 16.6 us; 64x260x346: 543 against
-// 132 us): returning atomics cost far more than the pass over the L2-resident grid they save.
+// 132 us): returning atomics cost far more than the pass over the L2-resident grid they save.  Rebuilt in round 2
+// with per-warp fp64 accumulators and measured again, then removed: 419 against 367 us at 64x480x640, 56 against
+// 30 us at 1x624x970 -- every add becomes a round trip its thread waits for.
 // Also measured and dropped: statistics + normalisation as ONE pass (a CTA keeps its <= 32 KB slice of a window in
 // registers, publishes its partial, waits on a per-window arrival counter -- tickets make the wait deadlock-free --
 // and normalises out of registers: one read, one write, one launch).  Parity-green but slower than the two
 // kernels at every shape (8x180x240: 18.7 against 16.6 us; 8x480x640: 55.2 against 43.6 us): the ticket atomic
 // sits in front of every load address and the waiting CTAs hold their SM slots idle.
+// Also measured and removed:
+//   - privatising the grid in the distributed shared memory of a thread-block cluster and scattering with
+//     red.shared::cluster.add.f32.  DSMEM atomics sustain ~19 G adds/s chip-wide vs ~69 G/s for L2 atomics on a
+//     B200, so that path was 2-4x SLOWER than the L2 one (timed with scripts/voxel_microbench.py).
+//   - the four L2 stages (zero, scatter, statistics, normalise) of four consecutive chunks fused horizontally into
+//     one launch per step: 573 against 365 us at 64x480x640, 78 against 43 us at 8x480x640 -- the stages did not
+//     overlap usefully inside one launch.
 // Time normalisation is fp64 with the reference's operation order
 // (mul, then div) in both modes, so bin assignment is identical.
-#include <cooperative_groups.h>
-#include <stdlib.h>
-
 #include "voxel_common.cuh"
-
-namespace cg = cooperative_groups;
 
 namespace cf {
 
 // ------------------------------------------------------------ atomic mode ---
 constexpr int kScatterThreads = 256;
 constexpr int kScatterUnroll = 4;
+constexpr size_t kL2ChunkBytes = (size_t)96 << 20;  // grids + events of one chunk of windows (of the B200's 126 MB L2)
 
-__device__ __forceinline__ void scatter_body(const double *__restrict__ ev, const int64_t *__restrict__ off,
-                                             int B, int nb, int H, int W, int flavour, float *__restrict__ out, int b_first,
-                                             int b_end, int blk, int nblk) {
+__global__ void __launch_bounds__(kScatterThreads)
+voxel_scatter_atomic_kernel(const double *__restrict__ ev, const int64_t *__restrict__ off,
+                            int B, int nb, int H, int W, int flavour, float *__restrict__ out, int b_first, int b_end) {
     // the events of windows [b_first, b_end) (one L2-sized chunk of the batch), grid-stride over
     // tiles of 1024 events: the host does not know the chunk's event count (offsets are on the device)
     const int64_t ev_first = __ldg(off + b_first), ev_end = __ldg(off + b_end);
@@ -66,7 +64,7 @@ __device__ __forceinline__ void scatter_body(const double *__restrict__ ev, cons
     constexpr int64_t kTileEvents = kScatterThreads * kScatterUnroll;
     Window w;
     w.b = -1;
-    for (int64_t tile = ev_first + (int64_t)blk * kTileEvents; tile < ev_end; tile += (int64_t)nblk * kTileEvents) {
+    for (int64_t tile = ev_first + (int64_t)blockIdx.x * kTileEvents; tile < ev_end; tile += (int64_t)gridDim.x * kTileEvents) {
         Event e[kScatterUnroll];
 #pragma unroll
         for (int k = 0; k < kScatterUnroll; ++k) {  // all loads in flight first
@@ -94,281 +92,6 @@ __device__ __forceinline__ void scatter_body(const double *__restrict__ ev, cons
             if (b.bin + 1 < nb) atomicAdd(cell + planes_per_bin * plane, wr);
         }
     }
-}
-
-__global__ void __launch_bounds__(kScatterThreads)
-voxel_scatter_atomic_kernel(const double *__restrict__ ev, const int64_t *__restrict__ off,
-                            int B, int nb, int H, int W, int flavour, float *__restrict__ out, int b_first, int b_end) {
-    scatter_body(ev, off, B, nb, H, W, flavour, out, b_first, b_end, (int)blockIdx.x, (int)gridDim.x);
-}
-
-// ---- scatter + statistics in one pass (std normalisation) ------------------------------------------------
-// The statistics pass of the L2 path reads every grid of the chunk once more (~100 us of the 370 at 64 x 480x640) only to
-// form sum, sum of squares and the count of non-zero cells of the hot-pixel-filtered grid.  With RETURNING atomics they
-// telescope out of the scatter: an add takes a cell from `old` to `old + w` (the SM repeats the L2's round-to-nearest add;
-// no subnormals occur: |w| >= 2^-53), and f(new) - f(old), f(new)^2 - f(old)^2, [f(new) != 0] - [f(old) != 0] summed over all
-// adds of a cell give f(final), f(final)^2 and [f(final) != 0] (f = the hot-pixel filter; every difference and square is
-// exact in fp64).  Returning atomics retire at 87 G/s against 105 G/s for RED (profiles/r02/atomics_l2_probe.txt): the
-// scatter gets ~20 % slower and the statistics pass disappears.  Per thread fp64 accumulators, reduced per warp, three
-// atomics per warp and window into the window's first Partial (zeroed by the host); the normalise kernel is unchanged.
-// MEASURED (B200, same box, us per launch incl. normalisation): 64 x 480x640 419 against 367 with the separate statistics pass,
-// 8 x 480x640 50 against 44, 1 x 624x970 (1 M events) 56 against 30, 64 x 180x240 54.5 against 52.5 -- the returned values
-// make every add a round trip the thread waits for (8 in flight per thread at 2 CTAs per SM), far below the 87 G/s the
-// probe reached with nothing else to do.  Kept as an experiment (CF_VOXEL_FLAGS bit5), parity-tested; not the default.
-struct TelAcc {
-    double s, q;
-    long long n;
-    int b;
-};
-__device__ __forceinline__ void tel_flush(TelAcc &a, Partial *__restrict__ tel, int tel_stride) {
-    // lanes of a warp nearly always hold the same window: one reduced update then, else every lane for itself
-    const unsigned full = 0xffffffffu;
-    const int b0 = __shfl_sync(full, a.b, 0);
-    if (__all_sync(full, a.b == b0)) {
-        const double s = warp_sum(a.s), q = warp_sum(a.q);
-        const long long n = warp_sum(a.n);
-        if ((threadIdx.x & 31) == 0 && b0 >= 0 && (s != 0.0 || q != 0.0 || n != 0)) {
-            Partial *p = tel + (size_t)b0 * tel_stride;
-            atomicAdd(&p->sum, s);
-            atomicAdd(&p->sumsq, q);
-            atomicAdd(reinterpret_cast<unsigned long long *>(&p->nnz), (unsigned long long)n);
-        }
-    } else if (a.b >= 0 && (a.s != 0.0 || a.q != 0.0 || a.n != 0)) {
-        Partial *p = tel + (size_t)a.b * tel_stride;
-        atomicAdd(&p->sum, a.s);
-        atomicAdd(&p->sumsq, a.q);
-        atomicAdd(reinterpret_cast<unsigned long long *>(&p->nnz), (unsigned long long)a.n);
-    }
-    a.s = 0.0; a.q = 0.0; a.n = 0;
-}
-
-__global__ void __launch_bounds__(kScatterThreads)
-voxel_scatter_stats_kernel(const double *__restrict__ ev, const int64_t *__restrict__ off, int B, int nb, int H, int W,
-                           int flavour, float *__restrict__ out, int b_first, int b_end, float hot_thr,
-                           Partial *__restrict__ tel, int tel_stride) {
-    const int blk = (int)blockIdx.x, nblk = (int)gridDim.x;
-    const int64_t ev_first = __ldg(off + b_first), ev_end = __ldg(off + b_end);
-    const int64_t plane = (int64_t)H * W;
-    const int planes_per_bin = flavour == CF_FLAVOUR_POL ? 2 : 1;
-    constexpr int64_t kTileEvents = kScatterThreads * kScatterUnroll;
-    Window w;
-    w.b = -1;
-    TelAcc acc{0.0, 0.0, 0, -1};
-    for (int64_t tile = ev_first + (int64_t)blk * kTileEvents; tile < ev_end; tile += (int64_t)nblk * kTileEvents) {
-        Event e[kScatterUnroll];
-#pragma unroll
-        for (int k = 0; k < kScatterUnroll; ++k) {  // all loads in flight first
-            const int64_t i = tile + k * kScatterThreads + threadIdx.x;
-            if (i < ev_end) e[k] = load_event(ev, i);
-        }
-        // all adds of the tile in flight before the first returned value is used
-        float *cell[kScatterUnroll];
-        float wl[kScatterUnroll], wr[kScatterUnroll], ol[kScatterUnroll], orr[kScatterUnroll];
-        int wb[kScatterUnroll];
-        bool two[kScatterUnroll];
-#pragma unroll
-        for (int k = 0; k < kScatterUnroll; ++k) {
-            const int64_t i = tile + k * kScatterThreads + threadIdx.x;
-            cell[k] = nullptr;
-            two[k] = false;
-            wb[k] = -1;
-            if (i >= ev_end) continue;
-            locate_window(w, i, off, ev, B);
-            const Binned b = bin_event(e[k], w, nb, H, W, flavour);
-            if (!b.ok) continue;
-            if (flavour == CF_FLAVOUR_TORCH) {
-                weights_f32(b, wl[k], wr[k]);
-            } else {
-                double dl, dr;
-                weights_wide(b, flavour, dl, dr);
-                wl[k] = (float)dl;
-                wr[k] = (float)dr;
-            }
-            cell[k] = out + (((int64_t)w.b * nb + b.bin) * planes_per_bin + b.chan) * plane + (int64_t)b.y * W + b.x;
-            two[k] = b.bin + 1 < nb;
-            wb[k] = w.b;
-            ol[k] = atomicAdd(cell[k], wl[k]);
-            if (two[k]) orr[k] = atomicAdd(cell[k] + planes_per_bin * plane, wr[k]);
-        }
-#pragma unroll
-        for (int k = 0; k < kScatterUnroll; ++k) {
-            const bool live = cell[k] != nullptr;
-            // (warp-uniform test first: the flush is a warp collective)
-            if (__any_sync(0xffffffffu, live && wb[k] != acc.b && acc.b >= 0)) tel_flush(acc, tel, tel_stride);
-            if (!live) continue;
-            acc.b = wb[k];
-            auto take = [&](float old, float add) {
-                const float fo = hot_filter(old, hot_thr), fn = hot_filter(__fadd_rn(old, add), hot_thr);
-                acc.s += (double)fn - (double)fo;
-                acc.q += (double)fn * (double)fn - (double)fo * (double)fo;
-                acc.n += (long long)(fn != 0.f) - (long long)(fo != 0.f);
-            };
-            take(ol[k], wl[k]);
-            if (two[k]) take(orr[k], wr[k]);
-        }
-    }
-    tel_flush(acc, tel, tel_stride);
-}
-
-// ----------------------------------------- atomic mode, cluster (smem) path ---
-// fp32 add into the shared memory of CTA `rank` of this cluster (DSMEM), no return value
-__device__ __forceinline__ void red_add_cluster(float *local_ptr, unsigned rank, float v) {
-    const uint32_t a = (uint32_t)__cvta_generic_to_shared(local_ptr);
-    uint32_t r;
-    asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(r) : "r"(a), "r"(rank));
-    asm volatile("red.relaxed.cluster.shared::cluster.add.f32 [%0], %1;" ::"r"(r), "f"(v) : "memory");
-}
-
-constexpr int kClusterThreads = 256;
-
-__global__ void __launch_bounds__(kClusterThreads)
-voxel_cluster_kernel(const double *__restrict__ ev, const int64_t *__restrict__ off, int B, int nb, int H, int W,
-                     int flavour, int preprocess, float hot_thr, float *__restrict__ out, int slice) {
-    cg::cluster_group cluster = cg::this_cluster();
-    const unsigned rank = cluster.block_rank(), CS = cluster.num_blocks();
-    extern __shared__ __align__(16) float sm[];          // [slice] grid slice, then one Partial
-    Partial *part = reinterpret_cast<Partial *>(sm + slice);
-    __shared__ Partial warp_part[kClusterThreads / 32];
-    __shared__ double s_a, s_inv;
-    __shared__ int s_identity;
-
-    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-    const int planes = flavour == CF_FLAVOUR_POL ? 2 : 1;
-    const int64_t plane = (int64_t)H * W;
-    const int cells = (int)((int64_t)nb * planes * plane);
-    const int my_first = (int)rank * slice;
-    const int valid = max(0, min(slice, cells - my_first));  // cells this CTA owns
-    const int n_clusters = gridDim.x / CS;
-
-    for (int b = blockIdx.x / CS; b < B; b += n_clusters) {
-        // ---- phase 0: clear the slice
-        for (int i = tid; i < slice / 4; i += kClusterThreads) reinterpret_cast<float4 *>(sm)[i] = make_float4(0.f, 0.f, 0.f, 0.f);
-        cluster.sync();
-
-        // ---- phase 1: this CTA's share of the window's events -> DSMEM scatter
-        const int64_t begin = __ldg(off + b), end = __ldg(off + b + 1);
-        if (end > begin) {
-            Window w;
-            w.b = b; w.begin = begin; w.end = end;
-            w.t0 = __ldg(ev + 4 * begin);
-            w.span = __dsub_rn(__ldg(ev + 4 * (end - 1)), w.t0);
-            if (w.span == 0.0) w.span = 1.0;
-            const int64_t per = (end - begin + CS - 1) / CS;
-            const int64_t s = begin + (int64_t)rank * per, e = min(end, s + per);
-            constexpr int U = 4;
-            for (int64_t i0 = s + tid; i0 < e; i0 += (int64_t)U * kClusterThreads) {
-                Event evs[U];
-#pragma unroll
-                for (int k = 0; k < U; ++k) {
-                    const int64_t i = i0 + (int64_t)k * kClusterThreads;
-                    if (i < e) evs[k] = load_event(ev, i);
-                }
-#pragma unroll
-                for (int k = 0; k < U; ++k) {
-                    const int64_t i = i0 + (int64_t)k * kClusterThreads;
-                    if (i >= e) break;
-                    const Binned bb = bin_event(evs[k], w, nb, H, W, flavour);
-                    if (!bb.ok) continue;
-                    float wl, wr;
-                    if (flavour == CF_FLAVOUR_TORCH) {
-                        weights_f32(bb, wl, wr);
-                    } else {
-                        double dl, dr;
-                        weights_wide(bb, flavour, dl, dr);
-                        wl = (float)dl;
-                        wr = (float)dr;
-                    }
-                    const int cell = (int)(((int64_t)bb.bin * planes + bb.chan) * plane + (int64_t)bb.y * W + bb.x);
-                    const unsigned own = (unsigned)cell / (unsigned)slice;
-                    red_add_cluster(sm + (cell - (int)own * slice), own, wl);
-                    if (bb.bin + 1 < nb) {
-                        const int cell2 = cell + (int)(planes * plane);
-                        const unsigned own2 = (unsigned)cell2 / (unsigned)slice;
-                        red_add_cluster(sm + (cell2 - (int)own2 * slice), own2, wr);
-                    }
-                }
-            }
-        }
-        cluster.sync();
-
-        // ---- phase 2: statistics of the slice, exchanged through DSMEM (fixed order => every
-        //      CTA of the cluster derives bit-identical mean / scale)
-        double a = 0.0, inv = 1.0;
-        bool identity = true;
-        if (preprocess != CF_PRE_NONE) {
-            double sum = 0.0, sumsq = 0.0;
-            long long nnz = 0;
-            float mn = INFINITY, mx = -INFINITY;
-            for (int i = tid; i < valid; i += kClusterThreads) {
-                const float v = hot_filter(sm[i], hot_thr);
-                sum += (double)v;
-                sumsq += (double)v * (double)v;
-                nnz += (v != 0.f);
-                mn = fminf(mn, v);
-                mx = fmaxf(mx, v);
-            }
-            sum = warp_sum(sum); sumsq = warp_sum(sumsq); nnz = warp_sum(nnz);
-            mn = warp_min(mn); mx = warp_max(mx);
-            if (lane == 0) warp_part[warp] = Partial{sum, sumsq, nnz, mn, mx};
-            __syncthreads();
-            if (tid == 0) {
-                Partial t = warp_part[0];
-                for (int k = 1; k < kClusterThreads / 32; ++k) {
-                    t.sum += warp_part[k].sum; t.sumsq += warp_part[k].sumsq; t.nnz += warp_part[k].nnz;
-                    t.mn = fminf(t.mn, warp_part[k].mn); t.mx = fmaxf(t.mx, warp_part[k].mx);
-                }
-                *part = t;
-            }
-            cluster.sync();
-            if (warp == 0) {
-                double ts = 0.0, tq = 0.0;
-                long long tn = 0;
-                float tmn = INFINITY, tmx = -INFINITY;
-                if ((unsigned)lane < CS) {
-                    const Partial *rp = cluster.map_shared_rank(part, lane);
-                    ts = rp->sum; tq = rp->sumsq; tn = rp->nnz; tmn = rp->mn; tmx = rp->mx;
-                }
-                ts = warp_sum(ts); tq = warp_sum(tq); tn = warp_sum(tn);
-                tmn = warp_min(tmn); tmx = warp_max(tmx);
-                if (lane == 0) {
-                    if (preprocess == CF_PRE_STD) {
-                        s_identity = tn == 0;
-                        const double mean = tn ? ts / (double)tn : 0.0;
-                        const double var = tn ? tq / (double)tn - mean * mean : 0.0;
-                        s_a = mean;
-                        s_inv = 1.0 / (sqrt(fmax(var, 0.0)) + 1e-8);
-                    } else {
-                        s_identity = 0;
-                        s_a = (double)tmn;
-                        s_inv = 1.0 / ((double)tmx - (double)tmn + 1e-8);
-                    }
-                }
-            }
-            __syncthreads();
-            a = s_a; inv = s_inv; identity = s_identity != 0;
-        }
-
-        // ---- phase 3: normalise the slice and write it once
-        auto norm = [&](float raw) -> float {
-            if (preprocess == CF_PRE_NONE) return raw;
-            const float v = hot_filter(raw, hot_thr);
-            if (identity) return v;
-            if (preprocess == CF_PRE_STD) return (v != 0.f) ? (float)(((double)v - a) * inv) : 0.f;
-            return (float)(((double)v - a) * inv);
-        };
-        float *o = out + (int64_t)b * cells + my_first;
-        if ((cells & 3) == 0) {
-            for (int i = tid; i < valid / 4; i += kClusterThreads) {
-                const float4 q = reinterpret_cast<const float4 *>(sm)[i];
-                st_cs4(reinterpret_cast<float4 *>(o) + i, make_float4(norm(q.x), norm(q.y), norm(q.z), norm(q.w)));
-            }
-        } else {
-            for (int i = tid; i < valid; i += kClusterThreads) st_cs(o + i, norm(sm[i]));
-        }
-        // the next window's phase-0 cluster.sync() orders these reads before any remote add
-        __syncthreads();
-    }
-    cluster.sync();  // no CTA may exit while a peer can still address its shared memory
 }
 
 // ------------------------------------------------------ deterministic mode ---
@@ -651,8 +374,10 @@ constexpr int kStatThreads = 256;
 
 // Both kernels: one CTA = one chunk of a window; a thread streams its float4s with 4 loads in flight.
 // (Round-1a sized them for 296 CTAs with one load in flight per thread: 43 of 70 us at 8 x 480x640.)
-__device__ __forceinline__ void stats_body(const float *__restrict__ grid, int64_t cells, int64_t chunk_len, float hot_thr,
-                                           Partial *__restrict__ partials, int chunks, int b, int c) {
+__global__ void __launch_bounds__(kStatThreads)
+voxel_stats_kernel(const float *__restrict__ grid, int64_t cells, int64_t chunk_len, float hot_thr,
+                   Partial *__restrict__ partials, int chunks) {
+    const int b = (int)blockIdx.y, c = (int)blockIdx.x;
     const float *g = grid + (int64_t)b * cells;
     const int64_t s = (int64_t)c * chunk_len, e = min(cells, s + chunk_len);
     // short fp32 partials per thread (a few dozen terms), promoted to fp64 across threads and chunks
@@ -704,14 +429,9 @@ __device__ __forceinline__ void stats_body(const float *__restrict__ grid, int64
 }
 
 __global__ void __launch_bounds__(kStatThreads)
-voxel_stats_kernel(const float *__restrict__ grid, int64_t cells, int64_t chunk_len, float hot_thr,
-                   Partial *__restrict__ partials, int chunks) {
-    stats_body(grid, cells, chunk_len, hot_thr, partials, chunks, (int)blockIdx.y, (int)blockIdx.x);
-}
-
-__device__ __forceinline__ void normalise_body(const float *in, float *out /* may alias in */, int64_t cells, int64_t chunk_len,
-                                               float hot_thr, int mode, const Partial *__restrict__ partials, int chunks,
-                                               int b, int c) {
+voxel_normalise_kernel(const float *in, float *out /* may alias in */, int64_t cells, int64_t chunk_len,
+                       float hot_thr, int mode, const Partial *__restrict__ partials, int chunks) {
+    const int b = (int)blockIdx.y, c = (int)blockIdx.x;
     const float *g = in + (int64_t)b * cells;
     float *o = out + (int64_t)b * cells;
     const int64_t s = (int64_t)c * chunk_len, e = min(cells, s + chunk_len);
@@ -792,51 +512,6 @@ __device__ __forceinline__ void normalise_body(const float *in, float *out /* ma
     }
 }
 
-__global__ void __launch_bounds__(kStatThreads)
-voxel_normalise_kernel(const float *in, float *out /* may alias in */, int64_t cells, int64_t chunk_len,
-                       float hot_thr, int mode, const Partial *__restrict__ partials, int chunks) {
-    normalise_body(in, out, cells, chunk_len, hot_thr, mode, partials, chunks, (int)blockIdx.y, (int)blockIdx.x);
-}
-
-// ---------------------------------------------------------- pipelined launches ---
-// The four stages of the L2-atomic path (zero, scatter, statistics, normalise) of FOUR consecutive window chunks in ONE
-// launch: CTAs [0, n_scatter) scatter chunk k, the next n_stats CTAs reduce chunk k-1, then chunk k-2 is normalised and
-// chunk k+1 zero-filled.  The stages bind on different units -- the scatter on the L2's atomic ALUs (~105 G RED/s,
-// profiles/r02/atomics_l2_probe.txt), the other three on L2 bandwidth -- and run back to back each of them left the
-// machine half idle plus a launch ramp and tail per kernel (4 launches per chunk).  B + 3 launches of this kernel
-// replace 4 B of the single-stage kernels; all chunks in flight stay L2-resident (the host sizes them).
-struct PipeStage {
-    int b0, nbat, ctas;   // windows [b0, b0 + nbat) of the batch, CTAs of this stage (0: idle)
-};
-__global__ void __launch_bounds__(kScatterThreads)
-voxel_pipeline_kernel(const double *__restrict__ ev, const int64_t *__restrict__ off, int B, int nb, int H, int W, int flavour,
-                      float *__restrict__ out, int64_t cells, int64_t chunk_len, int chunks, float hot_thr, int mode,
-                      Partial *__restrict__ partials, PipeStage scat, PipeStage stat, PipeStage norm, PipeStage zero) {
-    static_assert(kScatterThreads == kStatThreads, "one block size for all stages");
-    int blk = (int)blockIdx.x;
-    if (blk < scat.ctas) {
-        scatter_body(ev, off, B, nb, H, W, flavour, out, scat.b0, scat.b0 + scat.nbat, blk, scat.ctas);
-        return;
-    }
-    blk -= scat.ctas;
-    if (blk < stat.ctas) {
-        stats_body(out, cells, chunk_len, hot_thr, partials, chunks, stat.b0 + blk / chunks, blk % chunks);
-        return;
-    }
-    blk -= stat.ctas;
-    if (blk < norm.ctas) {
-        normalise_body(out, out, cells, chunk_len, hot_thr, mode, partials, chunks, norm.b0 + blk / chunks, blk % chunks);
-        return;
-    }
-    blk -= norm.ctas;
-    {
-        float4 *z = reinterpret_cast<float4 *>(out + (int64_t)zero.b0 * cells);   // cells % 4 == 0 (checked by the host)
-        const int64_t n4 = (int64_t)zero.nbat * cells / 4;
-        for (int64_t i = (int64_t)blk * kScatterThreads + threadIdx.x; i < n4; i += (int64_t)zero.ctas * kScatterThreads)
-            z[i] = make_float4(0.f, 0.f, 0.f, 0.f);
-    }
-}
-
 static void stat_geometry(int B, int64_t cells, int &chunks, int64_t &chunk_len) {
     // ~8 CTAs per SM over the batch, chunks of >= 2048 cells (2 float4 per thread), <= kMaxChunks per window
     int64_t want = ceil_div(8 * 148, B > 0 ? B : 1);
@@ -848,8 +523,9 @@ static void stat_geometry(int B, int64_t cells, int &chunks, int64_t &chunk_len)
     chunk_len = (chunk_len + 3) & ~(int64_t)3;  // keeps every chunk start 16-byte aligned
 }
 
-static int run_preprocess(const float *in, float *out, int B, int64_t cells, int preprocess, float hot_thr,
-                          void *ws, size_t ws_bytes, cudaStream_t stream, bool stats_done = false) {
+// statistics + normalisation of B grids; also used by the packed-event path (voxel_packed.cu)
+int run_preprocess(const float *in, float *out, int B, int64_t cells, int preprocess, float hot_thr, void *ws,
+                   size_t ws_bytes, cudaStream_t stream) {
     CF_REQUIRE(B <= 65535, CF_ERR_INVALID_ARG, "preprocess: B > 65535");
     CF_REQUIRE(ws && ws_bytes >= (size_t)B * kMaxChunks * sizeof(Partial), CF_ERR_WORKSPACE,
                "preprocess: workspace too small (%zu < %zu)", ws_bytes, (size_t)B * kMaxChunks * sizeof(Partial));
@@ -859,19 +535,11 @@ static int run_preprocess(const float *in, float *out, int B, int64_t cells, int
     stat_geometry(B, cells, chunks, chunk_len);
     Partial *partials = reinterpret_cast<Partial *>(ws);
     dim3 grid(chunks, B);
-    if (!stats_done) {   // (else the scatter left each window's totals in its first Partial, the others zero)
-        voxel_stats_kernel<<<grid, kStatThreads, 0, stream>>>(in, cells, chunk_len, hot_thr, partials, chunks);
-        CF_LAUNCH_CHECK("voxel_stats_kernel");
-    }
+    voxel_stats_kernel<<<grid, kStatThreads, 0, stream>>>(in, cells, chunk_len, hot_thr, partials, chunks);
+    CF_LAUNCH_CHECK("voxel_stats_kernel");
     voxel_normalise_kernel<<<grid, kStatThreads, 0, stream>>>(in, out, cells, chunk_len, hot_thr, preprocess, partials, chunks);
     CF_LAUNCH_CHECK("voxel_normalise_kernel");
     return CF_OK;
-}
-
-// statistics + normalisation for the packed-event path (voxel_packed.cu)
-int run_preprocess_shared(const float *in, float *out, int B, int64_t cells, int preprocess, float hot_thr, void *ws,
-                          size_t ws_bytes, cudaStream_t stream) {
-    return run_preprocess(in, out, B, cells, preprocess, hot_thr, ws, ws_bytes, stream);
 }
 
 // implemented in voxel_tiled.cu (CF_VOXEL_ATOMIC_TILED)
@@ -896,73 +564,6 @@ int launch_voxel_tiled(const double *events, const int64_t *offsets, int64_t tot
 // chip's 33 MB of shared memory, and the ~100 G/s of L2 atomics it avoids were not the bound once the
 // statistics/normalise kernels were given enough loads in flight.  So the L2 path is the default and the
 // tiled path stays selectable (and tested) for the next round's work on it.
-static int voxel_flags();
-static bool use_tiled(int64_t, int, int64_t) {
-    return (voxel_flags() & 8) != 0;              // experiments: CF_VOXEL_FLAGS=8 forces the tiled path
-}
-
-// CF_VOXEL_FLAGS (debug / experiments): bit5 = statistics telescoped out of a returning-atomics scatter, bit4 = pipelined launches (four stages of four chunks per launch), bit3 = force the tiled path,
-// bit2 = force the L2-atomic path, bit1 = use the cluster / DSMEM-atomics path, bit0 = do not chunk
-static int voxel_flags() {
-    static int flags = -1;
-    if (flags < 0) {
-        const char *e = getenv("CF_VOXEL_FLAGS");
-        flags = e ? atoi(e) : 0;
-    }
-    return flags;
-}
-
-// Returns CF_OK / an error, or 1 when the window grid does not fit a 16-CTA cluster's shared memory.
-static int launch_cluster_path(const double *events, const int64_t *offsets, int B, int nb, int H, int W, int flavour,
-                               int preprocess, float hot_thr, float *out, int64_t cells, cudaStream_t stream) {
-    constexpr size_t kMaxSlice = 200 * 1024;  // bytes of grid per CTA
-    if (cells * sizeof(float) > 16 * kMaxSlice || cells >= (1ll << 30)) return 1;
-    // smallest power-of-two cluster that holds the grid; grow it while the launch would leave SMs idle
-    int cs = 1;
-    while ((size_t)ceil_div(cells, cs) * sizeof(float) > kMaxSlice) cs *= 2;
-    const int sms = sm_count();
-    while (cs < 16 && (int64_t)B * cs * 2 <= sms && ceil_div(cells, cs * 2) >= 4096) cs *= 2;
-    if (const char *force = getenv("CF_VOXEL_CS")) {  // experiments: force the cluster size (must still fit)
-        const int f = atoi(force);
-        if (f >= cs && f <= 16 && (f & (f - 1)) == 0) cs = f; else if (f > 0 && f < cs) return 1;
-    }
-    const int slice = (int)((ceil_div(cells, cs) + 3) & ~(int64_t)3);
-    const size_t smem = (size_t)slice * sizeof(float) + sizeof(Partial);
-    int dev = 0;
-    CF_CUDA(cudaGetDevice(&dev));
-    static bool configured[64] = {};
-    if (!configured[dev & 63]) {
-        CF_CUDA(cudaFuncSetAttribute(voxel_cluster_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(kMaxSlice + 1024)));
-        CF_CUDA(cudaFuncSetAttribute(voxel_cluster_kernel, cudaFuncAttributeNonPortableClusterSizeAllowed, 1));
-        configured[dev & 63] = true;
-    }
-    const int per_sm = (int)((227 * 1024) / (smem + 1024));
-    int64_t max_clusters = (int64_t)(sms / cs) * (per_sm < 1 ? 1 : per_sm);
-    if (cs == 16) max_clusters = 8 * (per_sm < 1 ? 1 : per_sm);  // one 16-CTA cluster per GPC
-    if (max_clusters < 1) max_clusters = 1;
-    const int n_clusters = (int)(B < max_clusters ? B : max_clusters);
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3((unsigned)(n_clusters * cs));
-    cfg.blockDim = dim3(kClusterThreads);
-    cfg.dynamicSmemBytes = smem;
-    cfg.stream = stream;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeClusterDimension;
-    attr[0].val.clusterDim.x = (unsigned)cs;
-    attr[0].val.clusterDim.y = 1;
-    attr[0].val.clusterDim.z = 1;
-    cfg.attrs = attr;
-    cfg.numAttrs = 1;
-    cudaError_t e = cudaLaunchKernelEx(&cfg, voxel_cluster_kernel, events, offsets, B, nb, H, W, flavour, preprocess, hot_thr,
-                                       out, slice);
-    count_launch("voxel_cluster_kernel");
-    if (e != cudaSuccess) {
-        set_error("launch of voxel_cluster_kernel (cluster %d, %zu B smem) failed: %s", cs, smem, cudaGetErrorString(e));
-        return CF_ERR_CUDA;
-    }
-    return CF_OK;
-}
-
 static int radix_bits(uint64_t max_key) {
     int bits = 1;
     while (bits < 32 && (max_key >> bits) != 0) ++bits;
@@ -1034,12 +635,7 @@ extern "C" int cf_voxel_bin(const double *events, const int64_t *offsets, int64_
     cudaStream_t stream = (cudaStream_t)stream_;
     const int planes = flavour == CF_FLAVOUR_POL ? 2 : 1;
     const int64_t cells = (int64_t)nb * planes * H * W;
-    if (mode == CF_VOXEL_ATOMIC && (voxel_flags() & 2)) {  // experimental, see the file header
-        int rc = launch_cluster_path(events, offsets, B, nb, H, W, flavour, preprocess, hot_thr, out, cells, stream);
-        if (rc != 1) return rc;  // 1 = grid too large for the cluster path -> global path below
-    }
-    if (mode == CF_VOXEL_ATOMIC && !force_l2 && !(voxel_flags() & 4) && flavour != CF_FLAVOUR_MVSEC &&
-        (force_tiled || use_tiled(total, B, (int64_t)nb * planes * H * W))) {
+    if (force_tiled) {
         const size_t base = align_up(cf_preprocess_workspace_bytes(B, 0), 256);
         const size_t need = voxel_tiled_workspace_bytes(total, B, nb, H, W, flavour);
         if (need > 0 && total > 0) {
@@ -1047,9 +643,10 @@ extern "C" int cf_voxel_bin(const double *events, const int64_t *offsets, int64_
                        ws_bytes, base + need);
             const int rc = launch_voxel_tiled(events, offsets, total, B, nb, H, W, flavour, preprocess, hot_thr, out,
                                               reinterpret_cast<char *>(ws) + base, ws_bytes - base, stream);
-            if (rc != 1) return rc;  // 1 = geometry not covered -> L2-atomic path below
+            if (rc != 1) return rc;  // 1 = geometry not covered
         }
-        CF_REQUIRE(!force_tiled || total == 0, CF_ERR_UNSUPPORTED,
+        // an empty batch takes the L2-atomic path below (zero-fill + normalise)
+        CF_REQUIRE(total == 0, CF_ERR_UNSUPPORTED,
                    "cf_voxel_bin: CF_VOXEL_ATOMIC_TILED does not cover B=%d, %dx%d, nb=%d", B, H, W, nb);
     }
     if (mode == CF_VOXEL_ATOMIC) {
@@ -1057,8 +654,7 @@ extern "C" int cf_voxel_bin(const double *events, const int64_t *offsets, int64_
         // The host does not know the per-window event counts (offsets live on the device), so the
         // events of a chunk are budgeted with the batch average; kernels take device offsets.
         const size_t per_window = (size_t)cells * sizeof(float) + (size_t)(total / B + 1) * 32;
-        static const size_t budget_mb = [] { const char *e = getenv("CF_VOXEL_CHUNK_MB"); return e ? (size_t)atoi(e) : (size_t)96; }();
-        int chunk = (voxel_flags() & 1) ? B : (int)((budget_mb << 20) / per_window);
+        int chunk = (int)(kL2ChunkBytes / per_window);
         if (chunk < 1) chunk = 1;
         if (chunk > B) chunk = B;
         if (preprocess != CF_PRE_NONE) {
@@ -1066,53 +662,6 @@ extern "C" int cf_voxel_bin(const double *events, const int64_t *offsets, int64_
                        "cf_voxel_bin: workspace too small (%zu < %zu)", ws_bytes, (size_t)B * kMaxChunks * sizeof(Partial));
             CF_REQUIRE(aligned16(ws), CF_ERR_ALIGN, "cf_voxel_bin: workspace not 16-byte aligned");
         }
-        if ((voxel_flags() & 16) && (cells & 3) == 0 && total > 0 && aligned16(out)) {
-            // ---- pipelined (experiment, CF_VOXEL_FLAGS bit4; measured SLOWER than one stage per launch on the B200: 64 x 480x640
-            //      573 against 365 us, 8 x 480x640 78 against 43 us -- the stages do not overlap usefully inside one launch):
-            //      stage s of chunk k runs in launch k + s (voxel_pipeline_kernel).  Four chunks are in
-            //      flight (zeroed | being scattered into | being reduced | being normalised): size them so that all
-            //      four stay L2-resident
-            int pc = (voxel_flags() & 1) ? B : (int)((budget_mb << 20) / (4 * per_window));
-            if (pc < 1) pc = 1;
-            if (pc > B) pc = B;
-            const int nch = (int)ceil_div(B, pc);
-            int chunks = 1;
-            int64_t chunk_len = cells;
-            if (preprocess != CF_PRE_NONE) stat_geometry(pc, cells, chunks, chunk_len);
-            Partial *partials = reinterpret_cast<Partial *>(ws);
-            const int64_t cap = (int64_t)sm_count() * 8;
-            auto stage = [&](int k, bool on) {
-                PipeStage st{0, 0, 0};
-                if (on && k >= 0 && k < nch) {
-                    st.b0 = k * pc;
-                    st.nbat = B - st.b0 < pc ? B - st.b0 : pc;
-                }
-                return st;
-            };
-            for (int step = 0; step < nch + 3; ++step) {
-                PipeStage zero = stage(step, true), scat = stage(step - 1, true);
-                PipeStage stat = stage(step - 2, preprocess != CF_PRE_NONE), norm = stage(step - 3, preprocess != CF_PRE_NONE);
-                if (zero.nbat) {
-                    int64_t c = ceil_div((int64_t)zero.nbat * cells / 4, kScatterThreads * 8);
-                    zero.ctas = (int)(c > 2 * cap ? 2 * cap : (c < 1 ? 1 : c));
-                }
-                if (scat.nbat) {
-                    int64_t blocks = ceil_div(ceil_div(total * scat.nbat, B), kScatterThreads * kScatterUnroll);
-                    scat.ctas = (int)(blocks > cap ? cap : (blocks < 1 ? 1 : blocks));
-                }
-                if (stat.nbat) stat.ctas = stat.nbat * chunks;
-                if (norm.nbat) norm.ctas = norm.nbat * chunks;
-                const int grid = zero.ctas + scat.ctas + stat.ctas + norm.ctas;
-                if (grid == 0) continue;
-                voxel_pipeline_kernel<<<(unsigned)grid, kScatterThreads, 0, stream>>>(
-                    events, offsets, B, nb, H, W, flavour, out, cells, chunk_len, chunks, hot_thr, preprocess, partials, scat, stat,
-                    norm, zero);
-                CF_LAUNCH_CHECK("voxel_pipeline_kernel");
-            }
-            return CF_OK;
-        }
-        const bool telescope = preprocess == CF_PRE_STD && (voxel_flags() & 32) && ws != nullptr &&
-                               ws_bytes >= (size_t)B * kMaxChunks * sizeof(Partial);
         for (int b0 = 0; b0 < B; b0 += chunk) {
             const int nbat = B - b0 < chunk ? B - b0 : chunk;
             float *o = out + (size_t)b0 * cells;
@@ -1124,27 +673,14 @@ extern "C" int cf_voxel_bin(const double *events, const int64_t *offsets, int64_
                 const int64_t cap = (int64_t)sm_count() * 8;
                 if (blocks > cap) blocks = cap;
                 if (blocks < 1) blocks = 1;
-                if (telescope) {
-                    // statistics out of the scatter's returned values (std mode; experiment, CF_VOXEL_FLAGS bit5 -- measured slower)
-                    Partial *tel = reinterpret_cast<Partial *>(reinterpret_cast<char *>(ws) + (size_t)b0 * kMaxChunks * sizeof(Partial));
-                    int tchunks;
-                    int64_t tlen;
-                    stat_geometry(nbat, cells, tchunks, tlen);
-                    CF_CUDA(cudaMemsetAsync(tel, 0, sizeof(Partial) * (size_t)nbat * tchunks, stream));
-                    voxel_scatter_stats_kernel<<<(unsigned)blocks, kScatterThreads, 0, stream>>>(
-                        events, offsets, B, nb, H, W, flavour, out, b0, b0 + nbat, hot_thr, tel - (size_t)b0 * tchunks, tchunks);
-                    CF_LAUNCH_CHECK("voxel_scatter_stats_kernel");
-                } else {
-                    voxel_scatter_atomic_kernel<<<(unsigned)blocks, kScatterThreads, 0, stream>>>(
-                        events, offsets, B, nb, H, W, flavour, out, b0, b0 + nbat);
-                    CF_LAUNCH_CHECK("voxel_scatter_atomic_kernel");
-                }
+                voxel_scatter_atomic_kernel<<<(unsigned)blocks, kScatterThreads, 0, stream>>>(
+                    events, offsets, B, nb, H, W, flavour, out, b0, b0 + nbat);
+                CF_LAUNCH_CHECK("voxel_scatter_atomic_kernel");
             }
             if (preprocess != CF_PRE_NONE) {
                 if (int rc = run_preprocess(o, o, nbat, cells, preprocess, hot_thr,
                                             reinterpret_cast<char *>(ws) + (size_t)b0 * kMaxChunks * sizeof(Partial),
-                                            ws_bytes - (size_t)b0 * kMaxChunks * sizeof(Partial), stream,
-                                            /*stats_done=*/telescope && total > 0)) return rc;
+                                            ws_bytes - (size_t)b0 * kMaxChunks * sizeof(Partial), stream)) return rc;
             }
         }
         return CF_OK;

@@ -18,9 +18,9 @@
 
 namespace cf {
 
-// from voxel.cu: zero -> [scatter] -> statistics -> normalise-in-place, shared with the fp64 path
-int run_preprocess_shared(const float *in, float *out, int B, int64_t cells, int preprocess, float hot_thr, void *ws,
-                          size_t ws_bytes, cudaStream_t stream);
+// from voxel.cu: statistics -> normalise, shared with the fp64 path
+int run_preprocess(const float *in, float *out, int B, int64_t cells, int preprocess, float hot_thr, void *ws,
+                   size_t ws_bytes, cudaStream_t stream);
 
 namespace vp {
 constexpr int THREADS = 256;
@@ -144,7 +144,7 @@ extern "C" int cf_voxel_bin_packed(const void *packed, const int64_t *offsets, i
             reinterpret_cast<const uint2 *>(packed), offsets, B, nb, H, W, out);
         CF_LAUNCH_CHECK("voxel_scatter_packed_kernel");
     }
-    if (preprocess != CF_PRE_NONE) return run_preprocess_shared(out, out, B, cells, preprocess, hot_thr, ws, ws_bytes, stream);
+    if (preprocess != CF_PRE_NONE) return run_preprocess(out, out, B, cells, preprocess, hot_thr, ws, ws_bytes, stream);
     return CF_OK;
 }
 

@@ -1,4 +1,4 @@
-"""Voxel binning (+normalise) timing at several sizes; run with CF_VOXEL_FLAGS / CF_VOXEL_CS to compare paths."""
+"""Voxel binning (+normalise) timing at several sizes."""
 import os
 import sys
 
@@ -10,7 +10,6 @@ from cistaflow_b200 import synth
 
 dev = torch.device("cuda", 0)
 cases = [(8, 15000, 180, 240), (64, 15000, 180, 240), (64, 50000, 260, 346), (512, 50000, 260, 346), (8, 100000, 480, 640)]
-tag = f"flags={os.environ.get('CF_VOXEL_FLAGS', '0')} cs={os.environ.get('CF_VOXEL_CS', 'auto')}"
 for (B, n, H, W) in cases:
     reps = max(1, min(8, 64 // B))
     sets = []
@@ -38,5 +37,5 @@ for (B, n, H, W) in cases:
         torch.cuda.synchronize()
         us = a.elapsed_time(b) / 10 * 1e3
         nbytes = B * (32 * n + 4 * 5 * H * W)
-        print(f"{tag} B={B:4d} n={n:6d} {H}x{W} norm={mode_norm}: {us:9.1f} us  {nbytes / us / 1e3:8.1f} GB/s "
+        print(f"B={B:4d} n={n:6d} {H}x{W} norm={mode_norm}: {us:9.1f} us  {nbytes / us / 1e3:8.1f} GB/s "
               f"({nbytes / us / 1e3 / 6545 * 100:5.1f}% of HBM)  {B * n / us:8.1f} Mev/s")

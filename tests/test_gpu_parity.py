@@ -125,7 +125,7 @@ def test_voxel_batched_vs_sequential_oracle(cuda_device, n, h, w, batch, flavour
     assert np.array_equal(bits(det), bits(ref))
     det2 = cf.events_to_voxel_grid_batched(ev_d, off_d, 5, w, h, flavour=flavour, mode="deterministic").cpu().numpy()
     assert np.array_equal(bits(det), bits(det2)), "deterministic mode must be run-to-run identical"
-    for path, kernel in (("atomic_l2", ("voxel_scatter_atomic_kernel", "voxel_pipeline_kernel")), ("atomic_tiled", ("voxel_tile_kernel",)),
+    for path, kernel in (("atomic_l2", ("voxel_scatter_atomic_kernel",)), ("atomic_tiled", ("voxel_tile_kernel",)),
                          ("atomic", None)):
         atom = cf.events_to_voxel_grid_batched(ev_d, off_d, 5, w, h, flavour=flavour, mode=path).cpu().numpy()
         assert kernel is None or last_kernel() in kernel
@@ -165,7 +165,7 @@ def test_voxel_atomic_paths_ragged_batches(cuda_device, h, w, counts, path):
     off = np.concatenate([[0], np.cumsum(counts)]).astype(np.int64)
     ev_d, off_d = dev_t(ev, cuda_device), dev_t(off, cuda_device)
     raw = cf.events_to_voxel_grid_batched(ev_d, off_d, 5, w, h, flavour="numpy", mode=path).cpu().numpy()
-    assert last_kernel() in (("voxel_tile_kernel",) if path == "atomic_tiled" else ("voxel_scatter_atomic_kernel", "voxel_pipeline_kernel"))
+    assert last_kernel() in (("voxel_tile_kernel",) if path == "atomic_tiled" else ("voxel_scatter_atomic_kernel",))
     fused = cf.events_to_voxel_grid_batched(ev_d, off_d, 5, w, h, normalize="std", filter_hot_pixel=True,
                                             flavour="numpy", mode=path).cpu().numpy()
     pol = cf.events_to_voxel_grid_batched(ev_d, off_d, 5, w, h, flavour="pol", mode=path).cpu().numpy()

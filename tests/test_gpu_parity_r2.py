@@ -9,7 +9,7 @@ import cistaflow_b200 as cf
 from cistaflow_b200 import synth
 from oracle import explicit, ref_port
 
-from test_gpu_parity import assert_voxel_close, bits, dev_t
+from test_gpu_parity import assert_voxel_close, bits, dev_t, last_kernel
 
 pytestmark = pytest.mark.gpu
 
@@ -252,6 +252,50 @@ def test_out_of_grid_events_are_dropped_where_the_reference_wraps(cuda_device):
     assert abs(float(wrapped.sum()) - float(ours.sum())) > 1.0   # the wrapped events' polarity mass is in the reference grid only
 
 
+@pytest.mark.parametrize("mode", ["atomic", "atomic_l2"])
+def test_voxel_l2_path_over_several_chunks(cuda_device, mode):
+    """The L2-atomic path splits the batch into chunks of windows whose grids and events fit a 96 MB L2 budget, and the
+    statistics of a chunk go to its own slice of the workspace.  80 windows at 180x240 need two chunks: every window
+    against the sequential oracle, raw and with fused normalisation, with empty and ragged windows on both sides of
+    each flavour's chunk boundary."""
+    h, w, nb, B = 180, 240, 5, 80
+    specials = [0, 4099, 0, 3]                                   # per boundary: windows c-2, c-1 | c, c+1
+    counts = [15000] * (B - 2 * len(specials)) + 2 * specials
+    total = sum(counts)
+    bounds = {}
+    for flavour, planes in (("numpy", 1), ("pol", 2)):
+        per_window = nb * planes * h * w * 4 + (total // B + 1) * 32   # bytes per window of the chunk budget
+        chunk = (96 << 20) // per_window
+        assert -(-B // chunk) >= 2, (flavour, chunk)
+        bounds[flavour] = chunk
+    assert abs(bounds["numpy"] - bounds["pol"]) >= 2 * len(specials) and max(bounds.values()) + 2 <= B
+    special_at = {c + k: n for c in bounds.values() for k, n in zip((-2, -1, 0, 1), specials)}
+    counts = [special_at.get(i, 15000) for i in range(B)]
+    assert sum(counts) == total
+    wins = [synth.events(n, h, w, seed=900 + i) if n else np.zeros((0, 4)) for i, n in enumerate(counts)]
+    ev = np.concatenate(wins, axis=0)
+    off = np.concatenate([[0], np.cumsum(counts)]).astype(np.int64)
+    ev_d, off_d = dev_t(ev, cuda_device), dev_t(off, cuda_device)
+    for flavour, fl in (("numpy", explicit.FLAVOUR_NUMPY), ("pol", explicit.FLAVOUR_POL)):
+        raw = cf.events_to_voxel_grid_batched(ev_d, off_d, nb, w, h, flavour=flavour, mode=mode).cpu().numpy()
+        assert last_kernel() == "voxel_scatter_atomic_kernel"
+        fused = {}
+        for norm in ("std", "maxmin"):
+            fused[norm] = cf.events_to_voxel_grid_batched(ev_d, off_d, nb, w, h, normalize=norm, filter_hot_pixel=True,
+                                                          flavour=flavour, mode=mode).cpu().numpy()
+            assert last_kernel() == "voxel_normalise_kernel"
+        for b, win in enumerate(wins):
+            ref = explicit.voxel_grid_sequential(win, nb, w, h, fl)
+            mag = None
+            if flavour == "numpy":                                # the pol grid holds positive weights: |ref| is M
+                pos = win.copy()
+                pos[:, 3] = 1.0
+                mag = explicit.voxel_grid_sequential(pos, nb, w, h, fl)
+            assert_voxel_close(raw[b], ref, mag)
+            for norm, got in fused.items():
+                np.testing.assert_allclose(got[b], explicit.preprocess(ref, norm, 25.0 / nb), rtol=1e-4, atol=1e-4)
+
+
 # ------------------------------------------------- experiment paths stay correct ---
 def _run_with_env(code, env_extra):
     import os
@@ -261,43 +305,6 @@ def _run_with_env(code, env_extra):
     res = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, timeout=300, env=env,
                          cwd=os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
     return res
-
-
-def test_voxel_pipelined_launches_subprocess(cuda_device):
-    """CF_VOXEL_FLAGS bit4 (read once per process): the four L2-path stages of four consecutive chunks in one launch per
-    step (measured slower, kept selectable): same results as the default path -- bit-identical raw grids are not
-    expected (atomic order), the tolerance is the atomic mode's."""
-    code = """
-import numpy as np, torch
-import cistaflow_b200 as cf
-from cistaflow_b200 import synth, _lib
-from oracle import explicit
-dev = torch.device('cuda', 0)
-for (h, w, n, B, mb) in ((60, 80, 9000, 7, '1'), (180, 240, 15000, 5, '96')):
-    ev, off = synth.event_windows(B, n, h, w, seed=3)
-    e, o = torch.from_numpy(ev).to(dev), torch.from_numpy(off).to(dev)
-    raw = cf.events_to_voxel_grid_batched(e, o, 5, w, h, flavour='numpy', mode='atomic_l2').cpu().numpy()
-    assert _lib.load().cf_last_kernel().decode() == EXPECT_RAW, _lib.load().cf_last_kernel()
-    fused = cf.events_to_voxel_grid_batched(e, o, 5, w, h, normalize='std', filter_hot_pixel=True, flavour='numpy',
-                                            mode='atomic_l2').cpu().numpy()
-    assert _lib.load().cf_last_kernel().decode() == EXPECT_FUSED, _lib.load().cf_last_kernel()
-    for b in range(B):
-        ref = explicit.voxel_grid_sequential(ev[off[b]:off[b + 1]], 5, w, h, explicit.FLAVOUR_NUMPY)
-        pos = ev[off[b]:off[b + 1]].copy(); pos[:, 3] = 1.0
-        mag = explicit.voxel_grid_sequential(pos, 5, w, h, explicit.FLAVOUR_NUMPY)
-        assert (np.abs(raw[b] - ref) <= 1e-5 * (mag + 1)).all()
-        np.testing.assert_allclose(fused[b], explicit.preprocess(ref, 'std', 5.0), rtol=1e-4, atol=1e-4)
-print('PIPE_OK')
-"""
-    # a 1 MB chunk budget forces several chunks (stages of different chunks in one launch) at the small shape
-    for mb in ("1", "96"):
-        res = _run_with_env("EXPECT_RAW = EXPECT_FUSED = 'voxel_pipeline_kernel'\n" + code, {"CF_VOXEL_FLAGS": "16", "CF_VOXEL_CHUNK_MB": mb})
-        assert res.returncode == 0 and "PIPE_OK" in res.stdout, res.stdout + res.stderr
-    # bit5: statistics telescoped out of a scatter with returning atomics (no statistics pass)
-    for mb in ("1", "96"):
-        res = _run_with_env("EXPECT_RAW, EXPECT_FUSED = 'voxel_scatter_atomic_kernel', 'voxel_normalise_kernel'\n" + code,
-                            {"CF_VOXEL_FLAGS": "32", "CF_VOXEL_CHUNK_MB": mb})
-        assert res.returncode == 0 and "PIPE_OK" in res.stdout, res.stdout + res.stderr
 
 
 def test_corr_two_pass_conversion_and_lsu_stores_subprocess(cuda_device):
