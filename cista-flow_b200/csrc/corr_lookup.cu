@@ -283,17 +283,23 @@ static int launch_lookup_r4l4(const Pyramid &pyr, const float *coords, float *ou
     return CF_OK;
 }
 
+// dynamic shared memory of corr_lookup_kernel<qt>: the patches plus the clamped coordinates
+static size_t lookup_smem_bytes(int qt, int levels, int radius) {
+    const int P = 2 * radius + 2;
+    return ((size_t)qt * ((levels * P * P) | 1) + 2 * qt) * sizeof(float);
+}
+constexpr size_t kLookupSmemCap = 200 * 1024;
+
 template <int QT>
 static int launch_lookup(const Pyramid &pyr, const float *coords, float *out, int B, int N, int levels, int radius,
                          cudaStream_t stream) {
-    const int K = 2 * radius + 1, P = K + 1;
-    const size_t smem = ((size_t)QT * ((levels * P * P) | 1) + 2 * QT) * sizeof(float);
-    CF_REQUIRE(smem <= 200 * 1024, CF_ERR_INVALID_ARG, "cf_corr_lookup: levels*radius too large for shared memory");
+    const size_t smem = lookup_smem_bytes(QT, levels, radius);
+    CF_REQUIRE(smem <= kLookupSmemCap, CF_ERR_INVALID_ARG, "cf_corr_lookup: levels*radius too large for shared memory");
     int dev = 0;
     CF_CUDA(cudaGetDevice(&dev));
     static bool opt_in[64] = {};
     if (!opt_in[dev & 63]) {
-        CF_CUDA(cudaFuncSetAttribute(corr_lookup_kernel<QT>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
+        CF_CUDA(cudaFuncSetAttribute(corr_lookup_kernel<QT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kLookupSmemCap));
         opt_in[dev & 63] = true;
     }
     dim3 grid((unsigned)ceil_div(N, QT), B);
@@ -325,11 +331,14 @@ extern "C" int cf_corr_lookup(const float *const *pyramid, const float *coords, 
     }
     const int N = h * w;
     cudaStream_t stream = (cudaStream_t)stream_;
-    // 16 queries per CTA when the problem is small (more CTAs than SMs), else 32 (128-byte stores)
-    const bool small = (int64_t)B * ceil_div(N, 32) < 4 * (int64_t)sm_count();
     if (radius == 4 && levels == 4) {
         return launch_lookup_r4l4(pyr, coords, out, B, N, stream);
     }
-    return small ? launch_lookup<16>(pyr, coords, out, B, N, levels, radius, stream)
-                 : launch_lookup<32>(pyr, coords, out, B, N, levels, radius, stream);
+    // 16 queries per CTA when the problem is small (more CTAs than SMs), else 32 (128-byte stores) -- unless 32 queries'
+    // patches do not fit the shared memory (5 or 6 levels at radius 8).  Both do the same arithmetic per element, so the
+    // result does not depend on which one runs.
+    const bool small = (int64_t)B * ceil_div(N, 32) < 4 * (int64_t)sm_count();
+    return (small || lookup_smem_bytes(32, levels, radius) > kLookupSmemCap)
+               ? launch_lookup<16>(pyr, coords, out, B, N, levels, radius, stream)
+               : launch_lookup<32>(pyr, coords, out, B, N, levels, radius, stream);
 }

@@ -10,13 +10,15 @@
 //   the reference's 2x/(W-1)-1 normalisation and align_corners=True un-normalisation cancel).
 // Channel l*(2r+1)^2 + i*(2r+1) + j moves i along x (the transposed window, SURVEY F7).
 // One CTA = 16 queries of one batch item: patches (as in the forward kernel) and the queries' output
-// gradients are staged in shared memory, then thread <-> patch element / thread <-> (query, channel).
+// gradients are staged in shared memory, then thread <-> patch element / thread <-> (query, channel).  Where 16
+// queries' patches and gradients exceed the shared memory (6 levels at radius 8: 236 KB), a CTA takes 8 queries and
+// 32 threads share each query's channels.
 #include "common.cuh"
 
 namespace cf {
 namespace lb {
 constexpr int THREADS = 256;
-constexpr int QT = 16;
+constexpr size_t SMEM_CAP = 200 * 1024;
 
 struct Pyramid {
     const float *ptr[CF_CORR_MAX_LEVELS];
@@ -25,6 +27,7 @@ struct Pyramid {
     int W[CF_CORR_MAX_LEVELS];
 };
 
+template <int QT>
 __global__ void __launch_bounds__(THREADS)
 corr_lookup_backward_kernel(const __grid_constant__ Pyramid pyr, const float *__restrict__ coords,
                             const float *__restrict__ grad_out, float *__restrict__ grad_coords, int N, int levels, int r,
@@ -83,7 +86,7 @@ corr_lookup_backward_kernel(const __grid_constant__ Pyramid pyr, const float *__
                 ay += g * ((p10 - p00) * (1.f - fx) + (p11 - p01) * fx);
             }
         }
-        atomicAdd(&gacc[2 * qi], ax);       // shared memory, 16 threads per query
+        atomicAdd(&gacc[2 * qi], ax);       // shared memory, THREADS / QT threads per query
         atomicAdd(&gacc[2 * qi + 1], ay);
         __syncthreads();
         if (tid < QT && q0 + tid < N) {
@@ -146,18 +149,27 @@ extern "C" int cf_corr_lookup_backward(const float *grad_out, const float *const
         }
     }
     const int K = 2 * radius + 1, P = K + 1;
-    const size_t smem = ((size_t)lb::QT * (((levels * P * P) | 1) + ((levels * K * K) | 1)) + 4 * lb::QT) * sizeof(float);
-    CF_REQUIRE(smem <= 200 * 1024, CF_ERR_INVALID_ARG, "cf_corr_lookup_backward: levels*radius too large for shared memory");
+    auto smem_bytes = [&](int qt) {
+        return ((size_t)qt * (((levels * P * P) | 1) + ((levels * K * K) | 1)) + 4 * qt) * sizeof(float);
+    };
+    const int qt = smem_bytes(16) <= lb::SMEM_CAP ? 16 : 8;
+    const size_t smem = smem_bytes(qt);
+    CF_REQUIRE(smem <= lb::SMEM_CAP, CF_ERR_INVALID_ARG, "cf_corr_lookup_backward: levels*radius too large for shared memory");
     int dev = 0;
     CF_CUDA(cudaGetDevice(&dev));
     static bool opt_in[64] = {};
     if (!opt_in[dev & 63]) {
-        CF_CUDA(cudaFuncSetAttribute(lb::corr_lookup_backward_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
+        CF_CUDA(cudaFuncSetAttribute(lb::corr_lookup_backward_kernel<16>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)lb::SMEM_CAP));
+        CF_CUDA(cudaFuncSetAttribute(lb::corr_lookup_backward_kernel<8>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)lb::SMEM_CAP));
         opt_in[dev & 63] = true;
     }
-    dim3 grid((unsigned)ceil_div(N, lb::QT), (unsigned)B);
-    lb::corr_lookup_backward_kernel<<<grid, lb::THREADS, smem, stream>>>(pyr, coords, grad_out, grad_coords, N, levels, radius,
-                                                                         grad_pyramid ? 1 : 0);
+    dim3 grid((unsigned)ceil_div(N, qt), (unsigned)B);
+    if (qt == 16)
+        lb::corr_lookup_backward_kernel<16><<<grid, lb::THREADS, smem, stream>>>(pyr, coords, grad_out, grad_coords, N, levels,
+                                                                             radius, grad_pyramid ? 1 : 0);
+    else
+        lb::corr_lookup_backward_kernel<8><<<grid, lb::THREADS, smem, stream>>>(pyr, coords, grad_out, grad_coords, N, levels,
+                                                                            radius, grad_pyramid ? 1 : 0);
     CF_LAUNCH_CHECK("corr_lookup_backward_kernel");
     return CF_OK;
 }
