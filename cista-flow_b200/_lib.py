@@ -62,6 +62,11 @@ ALTCORR_SYMBOLS = {
     "cf_corr_alt_prepare": (_i, [_vp, _vp, _i, _i, _i, _i, _i, _i, _vp, _sz, _vp]),
     "cf_corr_alt_lookup": (_i, [_vp, _vp, _i, _i, _i, _i, _i, _i, _i, _vp, _vp]),
 }
+# every symbol include/cistaflow_det.h declares (the deterministic warp adjoint, compiled into the same library)
+DET_SYMBOLS = {
+    "cf_warp_backward_det_workspace_bytes": (_sz, [_i, _i, _i, _i, _i, _i]),
+    "cf_warp_backward_det": (_i, [_vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _f, _vp, _sz, _vp]),
+}
 
 _lock = threading.Lock()
 _lib = None
@@ -72,7 +77,7 @@ class CistaFlowError(RuntimeError):
 
 
 def load() -> ctypes.CDLL:
-    """dlopen the library and bind every symbol of both headers (no GPU needed)."""
+    """dlopen the library and bind every symbol of the three headers (no GPU needed)."""
     global _lib
     if _lib is not None:
         return _lib
@@ -84,7 +89,7 @@ def load() -> ctypes.CDLL:
                     f"`python cista-flow_b200/build.py` (or __graft_entry__.build()). "
                     f"There is no CPU / PyTorch fallback for the hot path.")
             lib = ctypes.CDLL(LIB_PATH)
-            for name, (res, args) in {**SYMBOLS, **ALTCORR_SYMBOLS}.items():
+            for name, (res, args) in {**SYMBOLS, **ALTCORR_SYMBOLS, **DET_SYMBOLS}.items():
                 fn = getattr(lib, name)  # AttributeError if the .so lacks a declared symbol
                 fn.restype, fn.argtypes = res, args
             _lib = lib

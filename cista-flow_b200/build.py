@@ -20,8 +20,8 @@ INCLUDE = os.path.join(ROOT, "include")
 LIB = os.path.join(HERE, "libcistaflow.so")
 STAMP = os.path.join(HERE, ".libcistaflow.stamp")
 
-HEADERS = ["cistaflow.h", "cistaflow_altcorr.h"]
-SOURCES = ["api.cu", "voxel.cu", "voxel_tiled.cu", "voxel_packed.cu", "warp.cu", "warp_tma.cu", "warp_backward.cu", "fwl.cu", "corr_lookup.cu", "corr_lookup_backward.cu", "corr_build.cu", "corr_build_tc.cu", "corr_alt.cu"]
+HEADERS = ["cistaflow.h", "cistaflow_altcorr.h", "cistaflow_det.h"]
+SOURCES = ["api.cu", "voxel.cu", "voxel_tiled.cu", "voxel_packed.cu", "warp.cu", "warp_tma.cu", "warp_backward.cu", "warp_backward_det.cu", "fwl.cu", "corr_lookup.cu", "corr_lookup_backward.cu", "corr_build.cu", "corr_build_tc.cu", "corr_alt.cu"]
 
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a",

@@ -12,7 +12,8 @@
 // One CTA = 16 queries of one batch item: patches (as in the forward kernel) and the queries' output
 // gradients are staged in shared memory, then thread <-> patch element / thread <-> (query, channel).  Where 16
 // queries' patches and gradients exceed the shared memory (6 levels at radius 8: 236 KB), a CTA takes 8 queries and
-// 32 threads share each query's channels.
+// 32 threads share each query's channels.  The threads of a query leave their partial coordinate gradients in shared
+// memory and the query's owner thread adds them in thread order: the sum order is fixed, the result reproducible.
 #include "common.cuh"
 
 namespace cf {
@@ -39,14 +40,13 @@ corr_lookup_backward_kernel(const __grid_constant__ Pyramid pyr, const float *__
     float *patch = smem;                        // [QT][PS]
     float *go = patch + (size_t)QT * PS;        // [QT][GS]
     float *cxy = go + (size_t)QT * GS;          // [QT][2]
-    float *gacc = cxy + 2 * QT;                 // [QT][2]
+    float *part = cxy + 2 * QT;                 // [THREADS][2] partial coordinate gradients
     const int tid = threadIdx.x, b = blockIdx.y, q0 = blockIdx.x * QT;
     const float *cb = coords + (size_t)b * 2 * N;
     if (tid < QT) {
         const int q = q0 + tid;
         cxy[2 * tid] = q < N ? fminf(fmaxf(__ldg(cb + q), -1.0e6f), 1.0e6f) : 0.f;
         cxy[2 * tid + 1] = q < N ? fminf(fmaxf(__ldg(cb + N + q), -1.0e6f), 1.0e6f) : 0.f;
-        gacc[2 * tid] = gacc[2 * tid + 1] = 0.f;
     }
     // output gradients of the CTA's queries: 16 consecutive queries of a channel are 64 contiguous bytes
     const float *gob = grad_out + (size_t)b * CT * N;
@@ -86,12 +86,17 @@ corr_lookup_backward_kernel(const __grid_constant__ Pyramid pyr, const float *__
                 ay += g * ((p10 - p00) * (1.f - fx) + (p11 - p01) * fx);
             }
         }
-        atomicAdd(&gacc[2 * qi], ax);       // shared memory, THREADS / QT threads per query
-        atomicAdd(&gacc[2 * qi + 1], ay);
+        part[2 * tid] = ax;
+        part[2 * tid + 1] = ay;
         __syncthreads();
-        if (tid < QT && q0 + tid < N) {
-            grad_coords[(size_t)b * 2 * N + q0 + tid] = gacc[2 * tid];
-            grad_coords[(size_t)b * 2 * N + N + q0 + tid] = gacc[2 * tid + 1];
+        if (tid < QT && q0 + tid < N) {   // threads tid, tid + QT, tid + 2 QT, ... hold this query's partials
+            float sx = 0.f, sy = 0.f;
+            for (int t = tid; t < THREADS; t += QT) {
+                sx += part[2 * t];
+                sy += part[2 * t + 1];
+            }
+            grad_coords[(size_t)b * 2 * N + q0 + tid] = sx;
+            grad_coords[(size_t)b * 2 * N + N + q0 + tid] = sy;
         }
     }
     // patch gradients: 2x2 correlation of the window of output gradients with the bilinear weights
@@ -150,7 +155,7 @@ extern "C" int cf_corr_lookup_backward(const float *grad_out, const float *const
     }
     const int K = 2 * radius + 1, P = K + 1;
     auto smem_bytes = [&](int qt) {
-        return ((size_t)qt * (((levels * P * P) | 1) + ((levels * K * K) | 1)) + 4 * qt) * sizeof(float);
+        return ((size_t)qt * (((levels * P * P) | 1) + ((levels * K * K) | 1)) + 2 * qt + 2 * lb::THREADS) * sizeof(float);
     };
     const int qt = smem_bytes(16) <= lb::SMEM_CAP ? 16 : 8;
     const size_t smem = smem_bytes(qt);

@@ -11,7 +11,8 @@
 // gradient multipliers once; per channel 4 tap loads (for grad_flow), 4 fp32 RED.ADD into grad_img
 // (resolved in L2) and, at the end, the pixel's flow gradient -- written, or added to the four
 // full-resolution flow pixels when the x0.5 down-sampling of e2v/e2v_model.py:190 is fused (its adjoint).
-// grad_img / grad_flow are zeroed here.  Sum order is unspecified (atomics), like ATen's CUDA backward.
+// grad_img / grad_flow are zeroed here.  Sum order is unspecified (atomics), like ATen's CUDA backward; the
+// fixed-order form, for torch.use_deterministic_algorithms(True), is warp_backward_det.cu.
 // Next step (not done): privatise grad_img tiles in shared memory and flush once per tile.
 #include "warp_common.cuh"
 
@@ -19,30 +20,6 @@ namespace cf {
 namespace wb {
 constexpr int THREADS = 256;
 constexpr int CPG = 32;   // channels per thread
-
-struct Pos {
-    int x0, y0;               // top-left tap (floor of the sample position)
-    float ax0, ax1, ay0, ay1; // ix - x0, (x0 + 1) - ix, ...
-    float mx, my;             // d(ix)/d(gx), d(iy)/d(gy) incl. reflection sign and clipping
-};
-
-// ATen reflect_coordinates_set_grad(v, 0, 2*(size-1)) + clip_coordinates_set_grad, after unnormalize (align_corners)
-__device__ __forceinline__ float source_index_set_grad(float g, int size, float &mult) {
-    const float unnorm = (float)(size - 1) / 2.f;
-    float v = ((g + 1.f) / 2.f) * (float)(size - 1);
-    float m = 1.f;
-    if (size == 1) { mult = 0.f; return 0.f; }
-    const float span = (float)(size - 1);
-    if (v < 0.f) { v = -v; m = -1.f; }
-    const float extra = fmodf(v, span);
-    const int flips = (int)floorf(v / span);
-    if (flips & 1) { v = span - extra; m = -m; } else { v = extra; }
-    // clip: gradient 0 on and beyond the borders
-    if (v <= 0.f) { v = 0.f; m = 0.f; }
-    else if (v >= span) { v = span; m = 0.f; }
-    mult = m * unnorm;
-    return v;
-}
 
 __global__ void __launch_bounds__(THREADS)
 warp_backward_kernel(const float *__restrict__ grad_out, const float *__restrict__ img, const float *__restrict__ flow,
@@ -55,14 +32,10 @@ warp_backward_kernel(const float *__restrict__ grad_out, const float *__restrict
     const int y = p / W, x = p - y * W;
     const float *fb = flow + (size_t)b * 2 * fH * fW;
     const float2 uv = flow_at(fb, x, y, W, fH, fW, half != 0, sy, sx, FlowLR{}, 0);
-    const float gx = 2.f * (((float)x + sign * uv.x) / (float)W - 0.5f);
-    const float gy = 2.f * (((float)y + sign * uv.y) / (float)H - 0.5f);
-    float mx, my;
-    const float ix = source_index_set_grad(gx, W, mx), iy = source_index_set_grad(gy, H, my);
-    const float fx0 = floorf(ix), fy0 = floorf(iy);
-    const int x0 = (int)fx0, y0 = (int)fy0;
-    const float ax1 = (fx0 + 1.f) - ix, ax0 = ix - fx0, ay1 = (fy0 + 1.f) - iy, ay0 = iy - fy0;
-    const bool xin1 = x0 + 1 < W, yin1 = y0 + 1 < H;   // x0, y0 are always inside after the clip
+    const GradPos q = grad_pos(uv.x, uv.y, x, y, H, W, sign);
+    const int x0 = q.x0, y0 = q.y0;
+    const float ax1 = q.ax1, ax0 = q.ax0, ay1 = q.ay1, ay0 = q.ay0, mx = q.mx, my = q.my;
+    const bool xin1 = q.xin1, yin1 = q.yin1;
     const int o00 = y0 * W + x0, o01 = o00 + 1, o10 = o00 + W, o11 = o10 + 1;
     const float w00 = ax1 * ay1, w01 = ax0 * ay1, w10 = ax1 * ay0, w11 = ax0 * ay0;
 
@@ -100,11 +73,9 @@ warp_backward_kernel(const float *__restrict__ grad_out, const float *__restrict
             atomicAdd(gfb + fplane + p, gv);
         } else {
             // adjoint of the x0.5 bilinear (align_corners=True) down-sampling: same taps / lambdas as flow_at()
-            const float fy = sy * (float)y, fx = sx * (float)x;
-            const int yy0 = min((int)fy, fH - 1), xx0 = min((int)fx, fW - 1);
-            const int yy1 = yy0 + (yy0 < fH - 1 ? 1 : 0), xx1 = xx0 + (xx0 < fW - 1 ? 1 : 0);
-            const float ly1 = fminf(fmaxf(fy - (float)yy0, 0.f), 1.f), lx1 = fminf(fmaxf(fx - (float)xx0, 0.f), 1.f);
-            const float ly0 = 1.f - ly1, lx0 = 1.f - lx1;
+            const HalfTaps t = half_taps(x, y, fH, fW, sy, sx);
+            const int yy0 = t.y0, yy1 = t.y1, xx0 = t.x0, xx1 = t.x1;
+            const float ly0 = t.ly0, ly1 = t.ly1, lx0 = t.lx0, lx1 = t.lx1;
 #pragma unroll
             for (int k = 0; k < 2; ++k) {
                 float *c = gfb + k * fplane;

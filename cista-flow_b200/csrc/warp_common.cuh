@@ -119,6 +119,66 @@ __device__ __forceinline__ Taps make_taps(float u, float v, int x, int y, int H,
     return t;
 }
 
+// ---- adjoint of the warp (warp_backward.cu: atomic splat, warp_backward_det.cu: sort + gather) -------------------
+// ATen reflect_coordinates_set_grad(v, 0, 2*(size-1)) + clip_coordinates_set_grad, after unnormalize (align_corners)
+__device__ __forceinline__ float source_index_set_grad(float g, int size, float &mult) {
+    const float unnorm = (float)(size - 1) / 2.f;
+    float v = ((g + 1.f) / 2.f) * (float)(size - 1);
+    float m = 1.f;
+    if (size == 1) { mult = 0.f; return 0.f; }
+    const float span = (float)(size - 1);
+    if (v < 0.f) { v = -v; m = -1.f; }
+    const float extra = fmodf(v, span);
+    const int flips = (int)floorf(v / span);
+    if (flips & 1) { v = span - extra; m = -m; } else { v = extra; }
+    // clip: gradient 0 on and beyond the borders
+    if (v <= 0.f) { v = 0.f; m = 0.f; }
+    else if (v >= span) { v = span; m = 0.f; }
+    mult = m * unnorm;
+    return v;
+}
+
+struct GradPos {
+    int x0, y0;               // top-left tap (floor of the sample position)
+    float ax0, ax1, ay0, ay1; // ix - x0, (x0 + 1) - ix, ...
+    float mx, my;             // d(ix)/d(gx), d(iy)/d(gy) incl. reflection sign and clipping
+    bool xin1, yin1;          // the right / lower taps are inside (x0, y0 always are after the clip)
+};
+
+// sample position of output pixel (x, y) for flow (u, v) with the gradient multipliers of the backward pass
+__device__ __forceinline__ GradPos grad_pos(float u, float v, int x, int y, int H, int W, float sign) {
+    const float gx = 2.f * (((float)x + sign * u) / (float)W - 0.5f);
+    const float gy = 2.f * (((float)y + sign * v) / (float)H - 0.5f);
+    GradPos q;
+    const float ix = source_index_set_grad(gx, W, q.mx), iy = source_index_set_grad(gy, H, q.my);
+    const float fx0 = floorf(ix), fy0 = floorf(iy);
+    q.x0 = (int)fx0;
+    q.y0 = (int)fy0;
+    q.ax1 = (fx0 + 1.f) - ix; q.ax0 = ix - fx0; q.ay1 = (fy0 + 1.f) - iy; q.ay0 = iy - fy0;
+    q.xin1 = q.x0 + 1 < W;
+    q.yin1 = q.y0 + 1 < H;
+    return q;
+}
+
+// taps and lambdas of the x0.5 bilinear (align_corners=True) down-sampling at output pixel (x, y): those of flow_at()
+struct HalfTaps {
+    int y0, y1, x0, x1;
+    float ly0, ly1, lx0, lx1;
+};
+__device__ __forceinline__ HalfTaps half_taps(int x, int y, int fH, int fW, float sy, float sx) {
+    HalfTaps t;
+    const float fy = sy * (float)y, fx = sx * (float)x;
+    t.y0 = min((int)fy, fH - 1);
+    t.x0 = min((int)fx, fW - 1);
+    t.y1 = t.y0 + (t.y0 < fH - 1 ? 1 : 0);
+    t.x1 = t.x0 + (t.x0 < fW - 1 ? 1 : 0);
+    t.ly1 = fminf(fmaxf(fy - (float)t.y0, 0.f), 1.f);
+    t.lx1 = fminf(fmaxf(fx - (float)t.x0, 0.f), 1.f);
+    t.ly0 = 1.f - t.ly1;
+    t.lx0 = 1.f - t.lx1;
+    return t;
+}
+
 // Taps that reproduce the input pixel (weights 1, 0, 0, 0): what the reference's `if not flow_final.any()` branch
 // returns (e2v/e2v_model.py:184-185).  Used when the device-side gate says the flow is all zero -- a zero flow is
 // NOT the identity under the reference's 2*(x/W-0.5) normalisation (SURVEY.md F6), hence the explicit branch.

@@ -36,6 +36,7 @@ reference, all deliberate:
 from __future__ import annotations
 
 import os
+import warnings
 
 import numpy as np
 import torch
@@ -43,7 +44,8 @@ import torch
 from . import _lib
 
 # 'atomic' (fast, <=1e-5 rel.) or 'deterministic' (bit-exact vs the reference's
-# sequential accumulation).  Override per call with mode=... or globally here.
+# sequential accumulation).  Override per call with mode=... or globally here;
+# torch.use_deterministic_algorithms(True) makes the default 'deterministic' (resolve_mode).
 DEFAULT_MODE = os.environ.get("CISTAFLOW_VOXEL_MODE", "atomic")
 
 _MODES = {"atomic": _lib.VOXEL_ATOMIC, "deterministic": _lib.VOXEL_DETERMINISTIC,
@@ -59,6 +61,14 @@ def _device() -> torch.device:
     if not torch.cuda.is_available():
         raise RuntimeError("cistaflow_b200 needs a CUDA device (B200); there is no CPU fallback")
     return torch.device("cuda", torch.cuda.current_device())
+
+
+def resolve_mode(mode: str | None) -> str:
+    """The voxel mode a call runs: an explicit ``mode`` wins; otherwise 'deterministic' while
+    ``torch.use_deterministic_algorithms(True)`` is in force, else ``DEFAULT_MODE``."""
+    if mode:
+        return mode
+    return "deterministic" if torch.are_deterministic_algorithms_enabled() else DEFAULT_MODE
 
 
 def _check_args(events, num_bins, width, height):
@@ -91,7 +101,7 @@ def events_to_voxel_grid_batched(events: torch.Tensor, offsets: torch.Tensor, nu
     events = events.contiguous()
     offsets = offsets.to(torch.int64).contiguous()
     B = offsets.numel() - 1
-    mode_id = _MODES[mode or DEFAULT_MODE]
+    mode_id = _MODES[resolve_mode(mode)]
     flav = _FLAVOURS[flavour]
     pre = _PRE[normalize]
     thr = 0.0
@@ -159,7 +169,16 @@ def events_to_voxel_grid_packed(packed: torch.Tensor, offsets: torch.Tensor, num
                                 normalize: str | None = None, filter_hot_pixel: bool = False,
                                 hot_threshold: float | None = None, out: torch.Tensor | None = None) -> torch.Tensor:
     """``events_to_voxel_grid_batched`` for packed events (int64/uint64 CUDA tensor [sum N_b]): reads 8 B per
-    event.  Atomic-mode numerics; polarity and the 25/nb hot-pixel default follow ``events_to_voxel_grid``."""
+    event.  Atomic-mode numerics; polarity and the 25/nb hot-pixel default follow ``events_to_voxel_grid``.
+    There is no deterministic form: under ``torch.use_deterministic_algorithms(True)`` it raises RuntimeError (warns
+    with ``warn_only=True``), as torch does for its ops without a deterministic implementation."""
+    if torch.are_deterministic_algorithms_enabled():
+        msg = ("events_to_voxel_grid_packed does not have a deterministic implementation (it accumulates with fp32 "
+               "atomics), but you set 'torch.use_deterministic_algorithms(True)'. Unpacked events through "
+               "events_to_voxel_grid_batched(..., mode='deterministic') are bit-exact.")
+        if not torch.is_deterministic_algorithms_warn_only_enabled():
+            raise RuntimeError(msg)
+        warnings.warn(msg)
     _lib.require_cuda(packed, "packed")
     _lib.require_cuda(offsets, "offsets")
     assert packed.dim() == 1 and packed.element_size() == 8

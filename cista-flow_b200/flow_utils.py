@@ -10,7 +10,8 @@ done inside the kernel).
 
 Autograd: ``warp`` (hence ``backWarp`` / ``forwardWarp`` / ``FrameWarp.warp_frame``) is differentiable
 w.r.t. both the image and the flow -- the backward is ``cf_warp_backward``, the bilinear splat (the
-reference trains through these modules, loss.py:147,336,398).  The fused ``warp_frame_and_codes`` step is
+reference trains through these modules, loss.py:147,336,398).  Under ``torch.use_deterministic_algorithms(True)``
+it is ``cf_warp_backward_det`` instead: the same gradients summed in a fixed order, bitwise reproducible.  The fused ``warp_frame_and_codes`` step is
 inference-only (the evaluation drivers run under ``torch.no_grad()``).
 """
 from __future__ import annotations
@@ -32,7 +33,8 @@ def _prep(t: torch.Tensor, name: str, allow_grad: bool = False) -> torch.Tensor:
 
 
 class _WarpFunction(torch.autograd.Function):
-    """cf_warp forward, cf_warp_backward (bilinear splat + flow gradient) backward."""
+    """cf_warp forward, cf_warp_backward (bilinear splat + flow gradient) backward; cf_warp_backward_det when
+    torch.are_deterministic_algorithms_enabled()."""
 
     @staticmethod
     def forward(ctx, img, flow, sign):
@@ -49,11 +51,21 @@ class _WarpFunction(torch.autograd.Function):
         grad_img = torch.empty_like(img) if need_img else None
         grad_flow = torch.empty_like(flow) if need_flow else None
         lib = _lib.load()
+        fH, fW = flow.shape[2], flow.shape[3]
         with torch.cuda.device(img.device):
-            rc = lib.cf_warp_backward(grad_out.data_ptr(), img.data_ptr(), flow.data_ptr(), _lib.ptr(grad_img),
-                                      _lib.ptr(grad_flow), B, C, H, W, flow.shape[2], flow.shape[3], ctx.sign,
-                                      _lib.stream_ptr(img.device))
-        _lib.check(rc, "cf_warp_backward")
+            if torch.are_deterministic_algorithms_enabled():
+                # torch.use_deterministic_algorithms(True): the sort + gather adjoint, no float atomics
+                name = "cf_warp_backward_det"
+                ws_bytes = lib.cf_warp_backward_det_workspace_bytes(B, C, H, W, fH, fW)
+                ws = _lib.workspace(ws_bytes, img.device)
+                rc = lib.cf_warp_backward_det(grad_out.data_ptr(), img.data_ptr(), flow.data_ptr(), _lib.ptr(grad_img),
+                                              _lib.ptr(grad_flow), B, C, H, W, fH, fW, ctx.sign, _lib.ptr(ws), ws_bytes,
+                                              _lib.stream_ptr(img.device))
+            else:
+                name = "cf_warp_backward"
+                rc = lib.cf_warp_backward(grad_out.data_ptr(), img.data_ptr(), flow.data_ptr(), _lib.ptr(grad_img),
+                                          _lib.ptr(grad_flow), B, C, H, W, fH, fW, ctx.sign, _lib.stream_ptr(img.device))
+        _lib.check(rc, name)
         return grad_img, grad_flow, None
 
 

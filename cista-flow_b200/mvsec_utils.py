@@ -15,6 +15,9 @@ summed in fp32 by one ``index_put_(accumulate=True)`` per bin.  All of that is `
 ``cf_voxel_bin``; this module only arranges the arguments.  The reference's ``temporal_bilinear=False`` branch is not
 mirrored: no caller uses it, and its bin edges (``tend = tstart + dt``, the whole duration) put every event in bin 0.
 
+``mode`` is that of ``events_to_voxel_grid_batched``: None means 'deterministic' under
+``torch.use_deterministic_algorithms(True)`` and ``event_process.DEFAULT_MODE`` otherwise.
+
 Results come back where the inputs lived (CPU tensors for CPU / NumPy inputs, like the reference) unless ``device``
 says otherwise.  Deliberate differences: out-of-range coordinates are dropped (the reference raises IndexError); a
 window whose events all share one time stamp uses dT = 1 (the reference divides by zero and returns NaN).
