@@ -635,8 +635,12 @@ corr_tc_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant
                     }
                     fence_async_smem();
                     __syncwarp();
-                    if (lane == 0 && mb * BM + 32 * quarter < p.N && !(p.ablate & 1)) {  // (rows below the volume: nothing to store)
-                        tma_store_3d(&tmap_c, buf, j0 + c0, mb * BM + 32 * quarter, b);
+                    if (lane == 0) {
+                        if (mb * BM + 32 * quarter < p.N && !(p.ablate & 1))   // (rows below the volume: nothing to store)
+                            tma_store_3d(&tmap_c, buf, j0 + c0, mb * BM + 32 * quarter, b);
+                        // one bulk group per chunk, empty when nothing was stored: the wait_read<1> above counts groups, and
+                        // a skipped commit let a chunk overwrite a buffer whose store was still reading it (the last query
+                        // tile's rows below the volume, then a store of the next tile: zeros in the earlier tile's box)
                         tma_store_commit();
                     }
                     ++chunk_count;

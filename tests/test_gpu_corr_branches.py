@@ -22,14 +22,13 @@ import torch
 
 import cistaflow_b200 as cf
 from cistaflow_b200 import _lib
+from guarded_buffers import assert_written_and_guarded, guarded
 
 pytestmark = pytest.mark.gpu
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 U11 = 2.0 ** -11     # unit roundoff of a TF32 / fp16 significand
 U24 = 2.0 ** -24     # unit roundoff of fp32
-GUARD = 64           # floats of NaN in front of and behind every output view
-NAN_BITS = 0x7FC00000
 
 
 def dev_t(a, device):
@@ -42,36 +41,6 @@ def last_kernel():
 
 def launch_count():
     return _lib.load().cf_launch_count()
-
-
-# ------------------------------------------------------------------------------------------------ output buffers ---
-def guarded(shapes, device, misalign=None):
-    """Views of the given shapes inside one NaN-filled float32 buffer, GUARD floats of NaN around each.  Views start
-    on 16-byte boundaries, except view ``misalign``, which starts one float later."""
-    offs, pos = [], GUARD
-    for k, s in enumerate(shapes):
-        o = pos + (1 if k == misalign else 0)
-        offs.append(o)
-        pos = -(-(o + math.prod(s)) // 4) * 4 + GUARD
-    buf = torch.full((pos,), float("nan"), dtype=torch.float32, device=device)
-    views = [buf[o:o + math.prod(s)].view(s) for o, s in zip(offs, shapes)]
-    return buf, views
-
-
-def assert_written_and_guarded(buf, views, what):
-    """Every element of every view written (no NaN left), every float outside the views unchanged."""
-    inside = torch.zeros(buf.numel(), dtype=torch.bool, device=buf.device)
-    base = buf.data_ptr()
-    for k, v in enumerate(views):
-        o = (v.data_ptr() - base) // 4
-        inside[o:o + v.numel()] = True
-        nan = torch.isnan(v)
-        if nan.any():
-            first = np.unravel_index(int(nan.reshape(-1).nonzero()[0]), tuple(v.shape))
-            raise AssertionError(f"{what}: view {k} has {int(nan.sum())} unwritten elements, first at {first}")
-    bits = buf.view(torch.int32)[~inside]
-    bad = bits != NAN_BITS
-    assert not bad.any(), f"{what}: {int(bad.sum())} guard floats overwritten"
 
 
 # ----------------------------------------------------------------------------------------- planner restatement ---
@@ -213,6 +182,7 @@ BUILD_ROWS = [
     Row("AUTO picks f16 (N=2048, B*N >= 19200)", 10, 256, 32, 64, 4, 4, 0, 0),
     Row("f16 b_sw64 + pair2", 4, 256, 20, 80, 4, 2, 0, 1),
     Row("stream_l0 (volume > 64 MB)", 8, 256, 36, 44, 4, 4, 0, 0),
+    Row("levels=1, rows below the volume in each item's last query tile", 8, 128, 20, 80, 1, 0, 0, 0),
 ]
 BUILD_CASES = [pytest.param(row, prec, id=f"{row.B}x{row.D}x{row.h}x{row.w}-L{row.levels}-{prec}")
                for row in BUILD_ROWS for prec in ("tf32", "3xtf32", "auto", "f16") if prec != "f16" or row.D % 128 == 0]
