@@ -68,6 +68,12 @@ DET_SYMBOLS = {
     "cf_warp_backward_det": (_i, [_vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _f, _vp, _sz, _vp]),
 }
 
+# every symbol include/cistaflow_half.h declares (the opt-in fp16 correlation pyramid, compiled into the same library)
+HALF_SYMBOLS = {
+    "cf_corr_build_half": (_i, [_vp, _vp, _i, _i, _i, _i, _i, ctypes.POINTER(_vp), _i, _vp, _sz, _vp]),
+    "cf_corr_lookup_half": (_i, [ctypes.POINTER(_vp), _vp, _i, _i, _i, _i, _i, _vp, _vp]),
+}
+
 _lock = threading.Lock()
 _lib = None
 
@@ -77,7 +83,7 @@ class CistaFlowError(RuntimeError):
 
 
 def load() -> ctypes.CDLL:
-    """dlopen the library and bind every symbol of the three headers (no GPU needed)."""
+    """dlopen the library and bind every symbol of the four headers (no GPU needed)."""
     global _lib
     if _lib is not None:
         return _lib
@@ -89,7 +95,7 @@ def load() -> ctypes.CDLL:
                     f"`python cista-flow_b200/build.py` (or __graft_entry__.build()). "
                     f"There is no CPU / PyTorch fallback for the hot path.")
             lib = ctypes.CDLL(LIB_PATH)
-            for name, (res, args) in {**SYMBOLS, **ALTCORR_SYMBOLS, **DET_SYMBOLS}.items():
+            for name, (res, args) in {**SYMBOLS, **ALTCORR_SYMBOLS, **DET_SYMBOLS, **HALF_SYMBOLS}.items():
                 fn = getattr(lib, name)  # AttributeError if the .so lacks a declared symbol
                 fn.restype, fn.argtypes = res, args
             _lib = lib

@@ -20,7 +20,7 @@ INCLUDE = os.path.join(ROOT, "include")
 LIB = os.path.join(HERE, "libcistaflow.so")
 STAMP = os.path.join(HERE, ".libcistaflow.stamp")
 
-HEADERS = ["cistaflow.h", "cistaflow_altcorr.h", "cistaflow_det.h"]
+HEADERS = ["cistaflow.h", "cistaflow_altcorr.h", "cistaflow_det.h", "cistaflow_half.h"]
 SOURCES = ["api.cu", "voxel.cu", "voxel_tiled.cu", "voxel_packed.cu", "warp.cu", "warp_tma.cu", "warp_backward.cu", "warp_backward_det.cu", "fwl.cu", "corr_lookup.cu", "corr_lookup_backward.cu", "corr_build.cu", "corr_build_tc.cu", "corr_alt.cu"]
 
 NVCC_FLAGS = [

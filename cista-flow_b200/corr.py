@@ -27,6 +27,34 @@ from . import _lib
 DEFAULT_PRECISION = os.environ.get("CISTAFLOW_CORR_PRECISION", "auto")
 _PREC = {"tf32": _lib.CORR_TF32, "fp32": _lib.CORR_FP32, "f16": _lib.CORR_F16, "auto": _lib.CORR_AUTO,
          "3xtf32": _lib.CORR_3XTF32}
+# Storage of the pyramid: "f32" (default) or "f16" (cf_corr_build_half: IEEE binary16, half the bytes; the lookup widens
+# each tap to fp32; inference-only).  The fp16 pyramid is a precision decision the caller takes; the default stays fp32.
+DEFAULT_STORAGE = os.environ.get("CISTAFLOW_CORR_STORAGE", "f32")
+_STORAGE = {"f32": torch.float32, "f16": torch.float16}
+
+
+def _storage(storage: str | None) -> str:
+    st = storage or DEFAULT_STORAGE
+    if st not in _STORAGE:
+        raise ValueError(f"correlation storage {st!r} is not one of {sorted(_STORAGE)}")
+    return st
+
+
+def _check_half(prec: str, D: int, h: int, w: int) -> None:
+    """The fp16 pyramid's preconditions (include/cistaflow_half.h), as ValueErrors naming the reason: no silent fp32."""
+    if prec in ("fp32", "3xtf32"):
+        raise ValueError(f"storage='f16' with precision {prec!r}: fp16 storage would lose its fp32 accuracy "
+                         f"(use 'tf32', 'f16' or 'auto')")
+    if D % 32 != 0:
+        raise ValueError(f"storage='f16' needs D % 32 == 0 (got D={D})")
+    if (h * w) % 8 != 0:
+        raise ValueError(f"storage='f16' needs h*w % 8 == 0 for a 16-byte row pitch of the fp16 volume (got {h}x{w})")
+
+
+def _check_no_grad(what: str, *tensors) -> None:
+    if torch.is_grad_enabled() and any(t.requires_grad for t in tensors):
+        raise RuntimeError(f"cistaflow_b200 {what} is inference-only: an input requires grad "
+                           f"(run under torch.no_grad(), or use the default fp32 storage, which is differentiable)")
 
 
 def coords_grid(batch, ht, wd, device=None):
@@ -41,33 +69,44 @@ def _prep(t: torch.Tensor, name: str) -> torch.Tensor:
 
 
 def build_pyramid(fmap1: torch.Tensor, fmap2: torch.Tensor, num_levels: int = 4, precision: str | None = None,
-                  out: list[torch.Tensor] | None = None):
+                  out: list[torch.Tensor] | None = None, storage: str | None = None):
+    """The correlation pyramid.  storage "f32" (default: CISTAFLOW_CORR_STORAGE, else "f32"): float32 levels
+    (cf_corr_build); "f16": float16 levels (cf_corr_build_half), which rejects precision "fp32" / "3xtf32" and shapes
+    without D % 32 == 0 and h*w % 8 == 0 with a ValueError."""
+    st = _storage(storage)
+    prec = precision or DEFAULT_PRECISION
+    if st == "f16":
+        _check_half(prec, *fmap1.shape[1:])
     fmap1, fmap2 = _prep(fmap1, "fmap1"), _prep(fmap2, "fmap2")
     assert fmap1.shape == fmap2.shape and fmap1.dim() == 4
     B, D, h, w = fmap1.shape
-    prec = precision or DEFAULT_PRECISION
     lib = _lib.load()
-    if prec in ("tf32", "f16", "auto", "3xtf32") and (D % 32 != 0 or (h * w) % 4 != 0):
+    if st == "f32" and prec in ("tf32", "f16", "auto", "3xtf32") and (D % 32 != 0 or (h * w) % 4 != 0):
         prec = "fp32"  # shapes the tensor-core tiling does not cover (never the model's: D=256, h,w % 4 == 0)
     dev = fmap1.device
     shapes = [(B * h * w, 1, h >> l, w >> l) for l in range(num_levels)]
+    dtype = _STORAGE[st]
     if out is None:
-        pyramid = [torch.empty(s, dtype=torch.float32, device=dev) for s in shapes]
+        pyramid = [torch.empty(s, dtype=dtype, device=dev) for s in shapes]
     else:
         pyramid = list(out)
         assert len(pyramid) == num_levels
         for t, s in zip(pyramid, shapes):
-            assert tuple(t.shape) == s and t.dtype == torch.float32 and t.is_contiguous() and t.device == dev
+            assert tuple(t.shape) == s and t.dtype == dtype and t.is_contiguous() and t.device == dev
+    build = lib.cf_corr_build_half if st == "f16" else lib.cf_corr_build
     with torch.cuda.device(dev):
         ws_bytes = lib.cf_corr_workspace_bytes(B, D, h, w, num_levels, _PREC[prec])
         ws = _lib.workspace(ws_bytes, dev)
-        rc = lib.cf_corr_build(fmap1.data_ptr(), fmap2.data_ptr(), B, D, h, w, num_levels, _lib.pointer_array(pyramid),
-                               _PREC[prec], _lib.ptr(ws), ws_bytes, _lib.stream_ptr(dev))
-    _lib.check(rc, "cf_corr_build")
+        rc = build(fmap1.data_ptr(), fmap2.data_ptr(), B, D, h, w, num_levels, _lib.pointer_array(pyramid),
+                   _PREC[prec], _lib.ptr(ws), ws_bytes, _lib.stream_ptr(dev))
+    _lib.check(rc, "cf_corr_build_half" if st == "f16" else "cf_corr_build")
     return pyramid
 
 
 def lookup(pyramid, coords: torch.Tensor, radius: int, out: torch.Tensor | None = None) -> torch.Tensor:
+    """cf_corr_lookup on a float32 pyramid, cf_corr_lookup_half on a float16 one (fp32 output either way)."""
+    half = pyramid[0].dtype == torch.float16
+    assert all(p.dtype == (torch.float16 if half else torch.float32) for p in pyramid), "pyramid levels of mixed dtypes"
     coords = _prep(coords, "coords")
     B, two, h, w = coords.shape
     assert two == 2
@@ -78,9 +117,10 @@ def lookup(pyramid, coords: torch.Tensor, radius: int, out: torch.Tensor | None 
         out = torch.empty((B, levels * k * k, h, w), dtype=torch.float32, device=coords.device)
     lib = _lib.load()
     with torch.cuda.device(coords.device):
-        rc = lib.cf_corr_lookup(_lib.pointer_array(pyramid), coords.data_ptr(), B, h, w, levels, radius, out.data_ptr(),
-                                _lib.stream_ptr(coords.device))
-    _lib.check(rc, "cf_corr_lookup")
+        fn = lib.cf_corr_lookup_half if half else lib.cf_corr_lookup
+        rc = fn(_lib.pointer_array(pyramid), coords.data_ptr(), B, h, w, levels, radius, out.data_ptr(),
+                _lib.stream_ptr(coords.device))
+    _lib.check(rc, "cf_corr_lookup_half" if half else "cf_corr_lookup")
     return out
 
 
@@ -93,7 +133,7 @@ class _PyramidFunction(torch.autograd.Function):
     @staticmethod
     def forward(ctx, fmap1, fmap2, num_levels, precision):
         ctx.save_for_backward(fmap1, fmap2)
-        pyramid = build_pyramid(fmap1, fmap2, num_levels, precision)
+        pyramid = build_pyramid(fmap1, fmap2, num_levels, precision, storage="f32")
         return tuple(pyramid)
 
     @staticmethod
@@ -150,18 +190,29 @@ class _LookupFunction(torch.autograd.Function):
 
 class CorrBlock:
     """Drop-in for ``ERAFT/corr.py:12-60`` / ``raft_corr.py:15-65``.  Differentiable like the reference's:
-    gradients reach the feature maps and the lookup coordinates when they are being recorded."""
+    gradients reach the feature maps and the lookup coordinates when they are being recorded.
 
-    def __init__(self, fmap1, fmap2, num_levels=4, radius=4, precision=None):
+    ``storage="f16"`` (or CISTAFLOW_CORR_STORAGE=f16) keeps ``corr_pyramid`` as float16 tensors: half the memory, the
+    reference's HalfCorrBlock choice.  That pyramid is inference-only (RuntimeError when an input requires grad while
+    gradients are recorded); ``CorrBlock.corr`` is unaffected."""
+
+    def __init__(self, fmap1, fmap2, num_levels=4, radius=4, precision=None, storage=None):
         self.num_levels = num_levels
         self.radius = radius
-        if torch.is_grad_enabled() and (fmap1.requires_grad or fmap2.requires_grad):
+        self.storage = _storage(storage)
+        if self.storage == "f16":
+            _check_no_grad("CorrBlock with storage='f16'", fmap1, fmap2)
+            with torch.no_grad():
+                self.corr_pyramid = build_pyramid(fmap1, fmap2, num_levels, precision, storage="f16")
+        elif torch.is_grad_enabled() and (fmap1.requires_grad or fmap2.requires_grad):
             self.corr_pyramid = list(_PyramidFunction.apply(_prep(fmap1, "fmap1"), _prep(fmap2, "fmap2"), num_levels, precision))
         else:
             with torch.no_grad():
-                self.corr_pyramid = build_pyramid(fmap1, fmap2, num_levels, precision)
+                self.corr_pyramid = build_pyramid(fmap1, fmap2, num_levels, precision, storage="f32")
 
     def __call__(self, coords):
+        if self.storage == "f16":
+            _check_no_grad("CorrBlock with storage='f16'", coords)
         if torch.is_grad_enabled() and (coords.requires_grad or any(p.requires_grad for p in self.corr_pyramid)):
             return _LookupFunction.apply(_prep(coords, "coords"), self.radius, *self.corr_pyramid)
         with torch.no_grad():
@@ -176,7 +227,7 @@ class CorrBlock:
             vol = _PyramidFunction.apply(_prep(fmap1, "fmap1"), _prep(fmap2, "fmap2"), 1, precision)[0]
         else:
             with torch.no_grad():
-                vol = build_pyramid(fmap1, fmap2, 1, precision)[0]
+                vol = build_pyramid(fmap1, fmap2, 1, precision, storage="f32")[0]
         return vol.view(B, h, w, 1, h, w)
 
 
