@@ -104,7 +104,9 @@ det_make_keys_kernel(const double *__restrict__ ev, const int64_t *__restrict__ 
                      uint32_t *__restrict__ keys, uint32_t *__restrict__ vals) {
     const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= total) return;
-    if (i >= __ldg(off + B)) {   // rows past the last window (a device-side filter kept fewer rows than the buffer holds)
+    // rows outside [off[0], off[B]) belong to no window: a row past the last one (a device-side filter kept fewer
+    // rows than the buffer holds), or a row before the first (offsets sliced from a longer stream, not rebased)
+    if (i < __ldg(off) || i >= __ldg(off + B)) {
         keys[i] = invalid_key;
         vals[i] = (uint32_t)i;
         return;
@@ -273,14 +275,15 @@ voxel_stats_kernel(const float *__restrict__ grid, int64_t cells, int64_t chunk_
     const int b = (int)blockIdx.y, c = (int)blockIdx.x;
     const float *g = grid + (int64_t)b * cells;
     const int64_t s = (int64_t)c * chunk_len, e = min(cells, s + chunk_len);
-    // short fp32 partials per thread (a few dozen terms), promoted to fp64 across threads and chunks
-    float fs = 0.f, fq = 0.f;
+    // fp64 partials per thread: a thread takes chunk_len / 256 terms, ~300 at 64 x 5x480x640 and thousands for
+    // larger batches, and fp32 running sums of a grid whose mean is large against its spread lose the variance
+    double fs = 0.0, fq = 0.0;
     int fn = 0;
     float mn = INFINITY, mx = -INFINITY;
     auto take = [&](float raw) {
         const float v = hot_filter(raw, hot_thr);
-        fs += v;
-        fq = fmaf(v, v, fq);
+        fs += (double)v;
+        fq = fma((double)v, (double)v, fq);   // the square of an fp32 value is exact in fp64
         fn += (v != 0.f);
         mn = fminf(mn, v);
         mx = fmaxf(mx, v);
@@ -304,7 +307,7 @@ voxel_stats_kernel(const float *__restrict__ grid, int64_t cells, int64_t chunk_
         for (int64_t i = s + threadIdx.x; i < e; i += kStatThreads) take(__ldg(g + i));
     }
     // fixed-shape tree: deterministic for a given launch geometry
-    double sum = warp_sum((double)fs), sumsq = warp_sum((double)fq);
+    double sum = warp_sum(fs), sumsq = warp_sum(fq);
     long long nnz = warp_sum((long long)fn);
     mn = warp_min(mn); mx = warp_max(mx);
     __shared__ Partial sh[kStatThreads / 32];
@@ -483,7 +486,8 @@ extern "C" size_t cf_preprocess_workspace_bytes(int B, int64_t) {
 extern "C" size_t cf_voxel_workspace_bytes(int64_t total_events, int B, int nb, int H, int W, int mode, int flavour, int) {
     size_t base = cf::align_up(cf_preprocess_workspace_bytes(B, 0), 256);
     if (mode == CF_VOXEL_DETERMINISTIC) return cf::det_layout(total_events, base).end;
-    if (mode != CF_VOXEL_ATOMIC_L2 && nb > 0 && H > 0 && W > 0)
+    // CF_VOXEL_ATOMIC runs the L2 path (cf_voxel_bin): only the forced tiled path needs its records and tables
+    if (mode == CF_VOXEL_ATOMIC_TILED && nb > 0 && H > 0 && W > 0)
         base += cf::voxel_tiled_workspace_bytes(total_events, B, nb, H, W, flavour);
     return base;
 }

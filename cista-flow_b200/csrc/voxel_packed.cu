@@ -5,6 +5,9 @@
 //                    rounding, so absolute stamps (~1e9 us, SURVEY F10) cost no precision
 //   word 1  uint32   x | y << 16 | p << 31          (x < 65536, y < 32768, p = 1 for positive polarity)
 //
+// A row outside [offsets[0], offsets[B]) belongs to no window: both packers write the invalid record for it
+// (x = 0xffff, t_rel = 0), and the voxel kernel does not visit it.
+//
 // cf_events_pack       device-side packer: fp64 rows -> packed (one pass, 32 B read + 8 B written per event)
 // cf_voxel_bin_packed  ATOMIC-mode voxel grid (+ fused event_preprocess) from packed events: the kernel
 //                      reads 8 B per event (4x fewer event bytes than cf_voxel_bin) and does the time
@@ -38,10 +41,15 @@ __device__ __forceinline__ int find_window(int64_t i, const int64_t *__restrict_
 __global__ void __launch_bounds__(THREADS)
 events_pack_kernel(const double *__restrict__ ev, const int64_t *__restrict__ off, int64_t total, int B,
                    uint2 *__restrict__ packed) {
+    const int64_t ev_first = __ldg(off), ev_end = __ldg(off + B);
     int b = -1;
     int64_t begin = 0, end = 0;
     double t0 = 0.0;
     for (int64_t i = (int64_t)blockIdx.x * THREADS + threadIdx.x; i < total; i += (int64_t)gridDim.x * THREADS) {
+        if (i < ev_first || i >= ev_end) {   // a row of no window: the invalid record (x = 0xffff, t_rel = 0)
+            packed[i] = make_uint2(0u, 0xffffu);
+            continue;
+        }
         const Event e = load_event(ev, i);
         if (b < 0 || i < begin || i >= end) {
             b = find_window(i, off, B);
@@ -61,13 +69,13 @@ events_pack_kernel(const double *__restrict__ ev, const int64_t *__restrict__ of
 __global__ void __launch_bounds__(THREADS)
 voxel_scatter_packed_kernel(const uint2 *__restrict__ packed, const int64_t *__restrict__ off, int B, int nb, int H, int W,
                             float *__restrict__ out) {
-    const int64_t ev_end = __ldg(off + B);
+    const int64_t ev_first = __ldg(off), ev_end = __ldg(off + B);   // rows outside the windows are not visited
     const int64_t plane = (int64_t)H * W;
     constexpr int64_t kTile = THREADS * UNROLL;
     int b = -1;
     int64_t begin = 0, end = 0;
     float span = 1.f;
-    for (int64_t tile = (int64_t)blockIdx.x * kTile; tile < ev_end; tile += (int64_t)gridDim.x * kTile) {
+    for (int64_t tile = ev_first + (int64_t)blockIdx.x * kTile; tile < ev_end; tile += (int64_t)gridDim.x * kTile) {
         uint2 e[UNROLL];
 #pragma unroll
         for (int k = 0; k < UNROLL; ++k) {  // all loads in flight first
@@ -274,7 +282,9 @@ __global__ void __launch_bounds__(256) window_offsets_kernel(const int64_t *__re
         k = (int64_t)rint((double)n / (double)param);
         if (k == 0) k = 1;
     }
-    if (k > max_windows) k = max_windows;    // (the caller sized the array; the last window then keeps the rest)
+    // the caller sized the array: FIXED keeps windows of `param` events and the last one keeps the rest; SPLIT splits
+    // the n events evenly over max_windows windows (np.array_split with k = max_windows)
+    if (k > max_windows) k = max_windows;
     const int64_t q = k > 0 ? n / k : 0, r = k > 0 ? n % k : 0;
     for (int i = blockIdx.x * blockDim.x + threadIdx.x; i <= max_windows; i += gridDim.x * blockDim.x) {
         int64_t o;

@@ -141,11 +141,14 @@ def pack_events_host(events: np.ndarray, offsets: np.ndarray | None = None) -> n
     for b in range(len(offsets) - 1):
         if offsets[b + 1] > offsets[b]:
             t0[offsets[b]:offsets[b + 1]] = ev[offsets[b], 0]
-    t_rel = (ev[:, 0] - t0).astype(np.float32).view(np.uint32).astype(np.uint64)
-    ok = (ev[:, 1] >= 0) & (ev[:, 1] < 65535) & (ev[:, 2] >= 0) & (ev[:, 2] < 32768)
+    # a row outside [offsets[0], offsets[B]) belongs to no window: the invalid record (x = 0xffff, t_rel = 0)
+    inside = np.zeros(n, dtype=bool)
+    inside[offsets[0]:offsets[-1]] = True
+    t_rel = np.where(inside, ev[:, 0] - t0, 0.0).astype(np.float32).view(np.uint32).astype(np.uint64)
+    ok = inside & (ev[:, 1] >= 0) & (ev[:, 1] < 65535) & (ev[:, 2] >= 0) & (ev[:, 2] < 32768)
     x = np.where(ok, ev[:, 1], 65535).astype(np.uint64)      # truncation like the kernels' (int) conversion
     y = np.where(ok, ev[:, 2], 0).astype(np.uint64)
-    p = (ev[:, 3] > 0).astype(np.uint64)
+    p = (inside & (ev[:, 3] > 0)).astype(np.uint64)
     return t_rel | ((x | (y << np.uint64(16)) | (p << np.uint64(31))) << np.uint64(32))
 
 

@@ -75,7 +75,7 @@ CF_API const char *cf_last_kernel(void);
  * ------------------------------------------------------------------------- */
 typedef enum cf_voxel_mode {
     CF_VOXEL_ATOMIC = 0,        /* fast: fp32 atomics, sum order unspecified (<= 1e-5 rel.);  */
-                                /* the library picks the data path (L2 or tiled) by size      */
+                                /* runs the L2 path (the tiled one only when forced, below)   */
     CF_VOXEL_DETERMINISTIC = 1, /* bit-exact: per-cell sums in the reference's event order    */
     CF_VOXEL_ATOMIC_L2 = 2,     /* ATOMIC, forced path: RED.ADD into the L2-resident grid     */
     CF_VOXEL_ATOMIC_TILED = 3   /* ATOMIC, forced path: partition + shared-memory tiles;      */
@@ -104,6 +104,9 @@ typedef enum cf_preprocess {
  *          fp64 is part of the contract: absolute stamps do not fit fp32
  *          (data_readers/event_readers.py:15-20, SURVEY.md F10).
  * offsets  int64 [B+1] (DEVICE), window b = rows [offsets[b], offsets[b+1]).
+ *          Rows outside [offsets[0], offsets[B]) belong to no window and are
+ *          ignored by every mode (offsets need not start at 0 nor end at
+ *          total_events).
  * out      float32 [B, nb, H, W]   (flavour POL: [B, nb, 2, H, W]).
  * hot_thr  > 0: entries with |v| > hot_thr are zeroed before the statistics
  *          (25/nb in event_preprocess, 20/nb in event_preprocess_pytorch);
@@ -111,6 +114,8 @@ typedef enum cf_preprocess {
  * Events whose (x, y) fall outside the grid are dropped (the reference would
  * raise IndexError; its callers pre-filter, data_readers/video_readers.py:208).
  * An empty window yields an all-zero grid (event_process.py:36-37).
+ * The window statistics of preprocess != NONE (sum, sum of squares, count)
+ * are accumulated in fp64; only the per-cell map is fp32.
  */
 CF_API size_t cf_voxel_workspace_bytes(int64_t total_events, int B, int nb, int H, int W,
                                 int mode, int flavour, int preprocess);
@@ -132,7 +137,9 @@ CF_API int cf_voxel_preprocess(const float *in, float *out, int B, int64_t cells
  *   word 0  float32 t_rel = (float)(t - t_first_of_window)   (fp64 subtraction first)
  *   word 1  uint32  x | y << 16 | p << 31                    (x < 65535, y < 32768)
  * ------------------------------------------------------------------------- */
-/* events float64 [total,4] + offsets int64 [B+1] (as cf_voxel_bin) -> packed uint64 [total]. */
+/* events float64 [total,4] + offsets int64 [B+1] (as cf_voxel_bin) -> packed uint64 [total].
+ * A row outside [offsets[0], offsets[B]) gets the invalid record (x = 0xffff, t_rel = 0), which
+ * cf_voxel_bin_packed never visits; pack_events_host writes the same bits. */
 CF_API int cf_events_pack(const double *events, const int64_t *offsets, int64_t total_events, int B,
                    void *packed, cf_stream_t stream);
 /* Device-side windowing (what data_readers/video_readers.py:208-232 and data_readers/event_readers.py:6-47 do on the host
@@ -143,6 +150,8 @@ CF_API int cf_events_pack(const double *events, const int64_t *offsets, int64_t 
  *   cf_event_window_offsets   offsets [max_windows+1] from a DEVICE-resident count:
  *                      CF_WINDOWS_FIXED  windows of `param` events, the last keeps the remainder (FixedSizeEventReader)
  *                      CF_WINDOWS_SPLIT  np.array_split into max(1, round(count / param)) windows (limit_num_events)
+ *                      more windows than max_windows: FIXED keeps max_windows windows of `param` events and the last
+ *                      keeps the rest; SPLIT splits the count evenly over max_windows windows;
  *                      entries past the last window = count (empty windows); *n_windows (device int, may be NULL). */
 enum cf_window_policy { CF_WINDOWS_FIXED = 0, CF_WINDOWS_SPLIT = 1 };
 CF_API size_t cf_events_filter_workspace_bytes(int64_t total_events);

@@ -73,7 +73,9 @@ def voxel_grid_sequential(events: np.ndarray, num_bins: int, width: int, height:
 def preprocess(grid: np.ndarray, mode: str = "std", hot_threshold: float = 0.0) -> np.ndarray:
     """utils/event_process.py:193-239 with the threshold passed explicitly
     (25/nb for the NumPy variant, 20/nb for the torch one, <= 0 disables).
-    Statistics in float64: the kernels accumulate them in fp64 as well."""
+    Statistics in float64: the kernels accumulate them in fp64 as well, per
+    thread and across threads (voxel_stats_kernel), or telescoped out of the
+    scatter (the tiled path); only their per-cell map is fp32."""
     g = np.array(grid, dtype=np.float32, copy=True)
     if hot_threshold > 0:
         g[np.abs(g) > F32(hot_threshold)] = 0
